@@ -27,6 +27,11 @@ Per record:
            host cores, rank 0.
 --impl reference times that same CPU port with all host threads (the reference's own CPU
 implementation is unbuildable here: no bazel / protoc / Eigen; DESIGN.md section 3).
+
+--dump-outputs DIR writes, per workload, what the last timed step handed back (the loss it
+fetched and the trained variables it left) as DIR/<workload>_<name>.npy in float32.  Inputs and
+initial weights are seeded, so two builds run with the same arguments can be compared array by
+array.
 """
 import argparse
 import ctypes
@@ -47,6 +52,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 METRIC = "Session.Run samples/sec (MLP-1024 & LeNet) at 1/2/4/8 B200 vs Eigen CPU"
 ALL_WORKLOADS = ["mlp", "lenet", "mlp_bf16"]
 MIN_WARMUP = 20   # steps; the first steps after a cold start run below the sustained clock
+DUMP_LIMIT_BYTES = 64 * 10**6   # all arrays of one --dump-outputs run together
 
 
 # =================================================================================== CPU arm
@@ -145,18 +151,15 @@ def run_reference(args):
         step, cores = cpu_step_fn(w)
         for _ in range(max(1, min(args.warmup, 2))):
             step()
-        # each step is a full training step of the workload; the run is bounded in time
-        steps, t0 = 0, time.perf_counter()
-        budget_s = 40.0 if name == "mlp" else 15.0
-        while steps < args.steps and (steps == 0 or time.perf_counter() - t0 < budget_s):
+        # each step is a full training step of the workload
+        steps, t0 = args.steps, time.perf_counter()
+        for _ in range(steps):
             step()
-            steps += 1
         dt = time.perf_counter() - t0
         value = w.batch * steps / dt
         gf = w.flops_per_step * steps / dt / 1e9
         note = ("CPU restatement of the reference's Eigen path, FMA build (reference unbuildable "
-                "offline: needs bazel+protoc+Eigen); %d of the requested %d steps ran inside the "
-                "%.0f s bound" % (steps, args.steps, budget_s))
+                "offline: needs bazel+protoc+Eigen)")
         if w.dtype == "bf16":
             note += ("; the reference has no bf16 MatMul on CPU (types.proto:30): this arm runs the "
                      "same graph in fp32")
@@ -317,6 +320,7 @@ class Bench:
             from simple_tensorflow_b200 import replica
             self.comm = replica.init_nccl_comm(self.L, self.rank, self.world, self.local_rank)
         self.peaks, self.peak_src = load_peaks()
+        self.outputs = {}   # --dump-outputs: name -> float32 array
 
     def collective_counts(self):
         p, n = ctypes.c_uint64(), ctypes.c_uint64()
@@ -388,6 +392,7 @@ class Bench:
             barrier()
             ms = ctypes.c_float()
             _lib.check(L.b200_event_elapsed_ms(ev0, ev1, ctypes.byref(ms)))
+            timed.last_loss = loss
             loss = float(np.asarray(w.to_f32(loss)).reshape(-1)[0])
             if world > 1:
                 import torch.distributed as dist
@@ -418,6 +423,11 @@ class Bench:
         ms_res, launches, loss_res = timed(res_fetch, None, args.steps)
         c1 = self.collective_counts()
         host_enqueue_us = timed.host_enqueue_us
+        if args.dump_outputs and rank == 0:
+            # read back before the passes below train the variables further
+            self.outputs["%s_loss" % name] = w.to_f32(timed.last_loss)
+            for n, a in zip(B.V, sess.run([v.ref for v in B.V.values()])):
+                self.outputs["%s_%s" % (name, n)] = w.to_f32(a)
         # the same K steps again in chunks: the median chunk is the figure robust to a cold start
         chunk = max(1, args.steps // 5)
         chunks = [timed(res_fetch, None, chunk)[0] / chunk for _ in range(5)] if args.steps >= 10 else []
@@ -516,6 +526,18 @@ class Bench:
         return rec
 
 
+def dump_outputs(directory, arrays):
+    """DIR/<name>.npy for every array, float32; refuses to write more than DUMP_LIMIT_BYTES."""
+    arrays = {n: np.ascontiguousarray(a, np.float32) for n, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d byte limit"
+                         % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(directory, n + ".npy"), a)
+
+
 def run_b200(args):
     # Libraries we load (NCCL's version banner) write to fd 1; the contract is ONE JSON line on
     # stdout, so everything else goes to stderr and the line is written to the saved descriptor.
@@ -530,6 +552,8 @@ def run_b200(args):
         import torch.distributed as dist
         dist.barrier()
     if b.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, b.outputs)
         head = args.workloads[0]
         line = dict(records[head])
         line["workloads"] = {n: r for n, r in records.items() if n != head}
@@ -551,12 +575,17 @@ def main():
                     help="comma list; the first is the line's top-level record (default: mlp = "
                          "BASELINE configs[1], then lenet = configs[2], mlp_bf16 = configs[3])")
     ap.add_argument("--workload", default=None, help="shorthand for --workloads <one>")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and trained variables of each workload's last timed step "
+                         "to DIR/<workload>_<name>.npy (float32)")
     args = ap.parse_args()
     args.workloads = [args.workload] if args.workload else [s for s in args.workloads.split(",") if s]
     for n in args.workloads:
         if n not in ALL_WORKLOADS:
             raise SystemExit("unknown workload %r (choose from %s)" % (n, ALL_WORKLOADS))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs dumps the GPU arm; it has no meaning with --impl reference")
         run_reference(args)
     else:
         run_b200(args)

@@ -3,9 +3,12 @@
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may
 import this module; the product package never does (tests/test_abi.py greps for that).
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -48,18 +51,33 @@ def _host_cpu():
 
 def build():
     """(Re)build oracle/_build/liboracle.so when it is missing, older than its source, or was
-    compiled (-march=native) on a different CPU model than the one we are running on."""
+    compiled (-march=native) on a different CPU model than the one we are running on.  In a
+    read-only tree (a benchmark run from an installed checkout) the rebuild goes to a temporary
+    directory instead."""
+    global ORACLE_SO, ORACLE_FAST_SO
     src = os.path.join(ORACLE_DIR, "oracle.c")
-    stamp = os.path.join(os.path.dirname(ORACLE_SO), "host.txt")
+    build_dir = os.path.dirname(ORACLE_SO)
+    stamp = os.path.join(build_dir, "host.txt")
     built_on = open(stamp).read().strip() if os.path.exists(stamp) else None
     foreign = built_on is not None and built_on != _host_cpu()
     stale = any((not os.path.exists(so)) or
                 (os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(so))
                 for so in (ORACLE_SO, ORACLE_FAST_SO))
-    if stale or foreign:
-        if foreign:
-            subprocess.check_call(["make", "-C", ORACLE_DIR, "clean"], stdout=subprocess.DEVNULL)
-        subprocess.check_call(["make", "-C", ORACLE_DIR], stdout=subprocess.DEVNULL)
+    if not (stale or foreign):
+        return
+    writable = os.access(build_dir if os.path.isdir(build_dir) else ORACLE_DIR, os.W_OK)
+    if not writable:
+        tmp = tempfile.mkdtemp(prefix="oracle-")
+        atexit.register(shutil.rmtree, tmp, True)
+        for f in ("Makefile", "oracle.c"):
+            shutil.copy(os.path.join(ORACLE_DIR, f), tmp)
+        subprocess.check_call(["make", "-C", tmp], stdout=subprocess.DEVNULL)
+        ORACLE_SO = os.path.join(tmp, "_build", "liboracle.so")
+        ORACLE_FAST_SO = os.path.join(tmp, "_build", "liboracle_fast.so")
+        return
+    if foreign:
+        subprocess.check_call(["make", "-C", ORACLE_DIR, "clean"], stdout=subprocess.DEVNULL)
+    subprocess.check_call(["make", "-C", ORACLE_DIR], stdout=subprocess.DEVNULL)
 
 
 def lib():
