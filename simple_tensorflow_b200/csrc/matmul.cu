@@ -388,17 +388,22 @@ int gemm_simt(const GemmArgs& g, cudaStream_t stream) {
   return check_launch("gemm_simt");
 }
 
-int gemm_dispatch(const GemmArgs& g, cudaStream_t stream) {
+// Tensor-core or CUDA-core kernel for this problem.  MatMul and the fused MatMul both ask here, so
+// adding a BiasAdd / Relu / ReluGrad tail never changes which kernel (and which arithmetic, TF32 or
+// IEEE fp32) computes the product.
+static bool use_tcgen05(const GemmArgs& g) {
   const bool want_exact = g.dtype == B200_DT_FLOAT && b200_get_matmul_precision() == 1;
   // Tiny problems: a 128-row MMA tile would be mostly padding and launch-bound anyway.
   const bool tiny = g.M * g.N * g.K < 32LL * 32 * 32;
   // matrix-vector / vector-matrix products: a 128-row MMA tile would be > 96 % padding; they are
   // bandwidth problems for the K-split CUDA-core kernel (exact fp32)
   const bool gemv_like = (g.N <= 4 && g.M >= 64) || (g.M <= 4 && g.N >= 64);
-  if (!want_exact && !tiny && !gemv_like && gemm_tcgen05_supported(g) &&
-      driver().cuTensorMapEncodeTiled)
-    return gemm_tcgen05(g, stream);
-  return gemm_simt(g, stream);
+  return !want_exact && !tiny && !gemv_like && gemm_tcgen05_supported(g) &&
+         driver().cuTensorMapEncodeTiled;
+}
+
+int gemm_dispatch(const GemmArgs& g, cudaStream_t stream) {
+  return use_tcgen05(g) ? gemm_tcgen05(g, stream) : gemm_simt(g, stream);
 }
 
 static int validate_gemm(const char* what, int dtype, const void* a, const void* b, void* c,
@@ -503,10 +508,9 @@ int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void* c, int64
     g.workspace = workspace;  // enables split-K; the bias / relu tail moves to the reduction pass
     g.workspace_bytes = workspace_bytes;
   }
-  const bool want_exact = dtype == B200_DT_FLOAT && b200_get_matmul_precision() == 1;
-  if (!want_exact && gemm_tcgen05_supported(g) && driver().cuTensorMapEncodeTiled)
-    return gemm_tcgen05(g, as_stream(stream));
-  // Shapes TMA cannot address / exact mode: GEMM, then the element-wise tail as separate kernels.
+  if (use_tcgen05(g)) return gemm_tcgen05(g, as_stream(stream));
+  // CUDA-core shapes (TMA cannot address them, tiny, matrix-vector) and exact mode: GEMM, then the
+  // element-wise tail as separate kernels.
   rc = gemm_simt(g, as_stream(stream));
   if (rc) return rc;
   if (bias) rc = b200_bias_add(dtype, c, bias, c, m, n, stream);

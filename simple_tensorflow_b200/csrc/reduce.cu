@@ -923,23 +923,28 @@ reduce_rows_kernel(const T* __restrict__ in, T* __restrict__ out, long long redu
 }
 template <typename T>
 __global__ void __launch_bounds__(256)
-reduce_mid_kernel(const T* __restrict__ in, T* __restrict__ out, long long reduce, long long inner,
-                  float scale) {
+reduce_mid_kernel(const T* __restrict__ in, T* __restrict__ out, long long outer, long long reduce,
+                  long long inner, float scale) {
   pdl_prologue();
   __shared__ float sm[8][32];
   const int x = threadIdx.x & 31, y = threadIdx.x >> 5;
   const long long col = (long long)blockIdx.x * 32 + x;
-  const T* base = in + (long long)blockIdx.y * reduce * inner;
-  float acc = 0.f;
-  if (col < inner)
-    for (long long r = y; r < reduce; r += 8) acc += ldf<T>(base + r * inner + col);
-  sm[y][x] = acc;
-  __syncthreads();
-  if (y == 0 && col < inner) {
-    float t = 0.f;
+  // grid-stride over `outer` (gridDim.y is capped at 65535); each (outer, column) is summed in the
+  // same order whatever the grid
+  for (long long o = blockIdx.y; o < outer; o += gridDim.y) {
+    const T* base = in + o * reduce * inner;
+    float acc = 0.f;
+    if (col < inner)
+      for (long long r = y; r < reduce; r += 8) acc += ldf<T>(base + r * inner + col);
+    __syncthreads();  // the previous row's merge has read sm
+    sm[y][x] = acc;
+    __syncthreads();
+    if (y == 0 && col < inner) {
+      float t = 0.f;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) t += sm[i][x];
-    stf<T>(out + (long long)blockIdx.y * inner + col, t * scale);
+      for (int i = 0; i < 8; ++i) t += sm[i][x];
+      stf<T>(out + o * inner + col, t * scale);
+    }
   }
 }
 template <typename T>
@@ -950,8 +955,9 @@ static int launch_reduce(const void* in, void* out, long long outer, long long r
   if (inner == 1) {
     launch_pdl(reduce_rows_kernel<T>, dim3((unsigned)outer), dim3(256), 0, s, x, y, reduce, scale);
   } else {
-    launch_pdl(reduce_mid_kernel<T>, dim3((unsigned)((inner + 31) / 32), (unsigned)outer), dim3(256),
-               0, s, x, y, reduce, inner, scale);
+    const unsigned gy = (unsigned)std::min<long long>(outer, 65535);
+    launch_pdl(reduce_mid_kernel<T>, dim3((unsigned)((inner + 31) / 32), gy), dim3(256), 0, s, x, y,
+               outer, reduce, inner, scale);
   }
   return B200_OK;
 }
@@ -1366,7 +1372,7 @@ int b200_reduce(int dtype, const void* in, void* out, int64_t outer, int64_t red
     return B200_UNIMPLEMENTED;
   }
   if (outer == 0 || inner == 0) return B200_OK;  // empty output
-  if (outer > 0x7fffffffLL || (inner + 31) / 32 > 0x7fffffffLL || (inner > 1 && outer > 65535)) {
+  if (outer > 0x7fffffffLL || (inner + 31) / 32 > 0x7fffffffLL) {
     set_last_error("b200_reduce: extent beyond the launch grid (outer %lld, inner %lld)",
                    (long long)outer, (long long)inner);
     return B200_UNIMPLEMENTED;

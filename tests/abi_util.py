@@ -65,7 +65,24 @@ def cdt(bf16):
     return _lib.DT_BFLOAT16 if bf16 else _lib.DT_FLOAT
 
 
-def matmul(a, b, ta=False, tb=False, bf16=False, use_workspace=True):
+def launches(fn, *args, **kwargs):
+    """(fn(*args, **kwargs), kernels libb200tf.so launched during the call)."""
+    L = lib()
+    before = L.b200_launch_count()
+    r = fn(*args, **kwargs)
+    return r, L.b200_launch_count() - before
+
+
+def offset_copy(a, bf16=False, offset=0):
+    """Device copy of `a` that starts `offset` elements into its allocation (offset 1: a pointer
+    that is NOT 16-byte aligned, every element still inside the allocation).  Returns (tensor, ptr)."""
+    flat = np.ascontiguousarray(a, np.float32).ravel()
+    t = dev(np.concatenate([np.zeros(offset, np.float32), flat]), bf16)
+    return t, t.data_ptr() + offset * t.element_size()
+
+
+def matmul(a, b, ta=False, tb=False, bf16=False, use_workspace=True, workspace_bytes=None):
+    """workspace_bytes: scratch size to pass (default: what b200_matmul_workspace_bytes asks for)."""
     L = lib()
     m = a.shape[1] if ta else a.shape[0]
     k = a.shape[0] if ta else a.shape[1]
@@ -73,6 +90,8 @@ def matmul(a, b, ta=False, tb=False, bf16=False, use_workspace=True):
     da, db = dev(a, bf16), dev(b, bf16)
     out = empty((m, n), tdt(bf16), fill=float("nan"))
     nb = L.b200_matmul_workspace_bytes(cdt(bf16), m, n, k) if use_workspace else 0
+    if workspace_bytes is not None:
+        nb = workspace_bytes
     w = ws(nb)
     call(L.b200_matmul, cdt(bf16), da.data_ptr(), db.data_ptr(), out.data_ptr(), m, n, k, int(ta),
          int(tb), w.data_ptr() if nb else None, nb, stream())
@@ -91,6 +110,28 @@ def fused_matmul(a, b, ta=False, tb=False, bias=None, relu=False, features=None,
     call(L.b200_fused_matmul, cdt(bf16), da.data_ptr(), db.data_ptr(), out.data_ptr(), m, n, k,
          int(ta), int(tb), dbias.data_ptr() if dbias is not None else None, int(relu),
          dfeat.data_ptr() if dfeat is not None else None, stream())
+    return host(out)
+
+
+def fused_matmul_ws(a, b, ta=False, tb=False, bias=None, relu=False, features=None, bf16=False,
+                    workspace_bytes=None, bias_offset=0):
+    """b200_fused_matmul_ws.  workspace_bytes: None = b200_matmul_workspace_bytes, 0 = no scratch.
+    bias_offset: elements between the bias allocation and the pointer passed (1: unaligned bias)."""
+    L = lib()
+    m = a.shape[1] if ta else a.shape[0]
+    k = a.shape[0] if ta else a.shape[1]
+    n = b.shape[0] if tb else b.shape[1]
+    da, db = dev(a, bf16), dev(b, bf16)
+    pbias = None
+    if bias is not None:
+        dbias, pbias = offset_copy(bias, bf16, bias_offset)
+    dfeat = dev(features, bf16) if features is not None else None
+    out = empty((m, n), tdt(bf16), fill=float("nan"))
+    nb = L.b200_matmul_workspace_bytes(cdt(bf16), m, n, k) if workspace_bytes is None else workspace_bytes
+    w = ws(nb)
+    call(L.b200_fused_matmul_ws, cdt(bf16), da.data_ptr(), db.data_ptr(), out.data_ptr(), m, n, k,
+         int(ta), int(tb), pbias, int(relu), dfeat.data_ptr() if dfeat is not None else None,
+         w.data_ptr() if nb else None, nb, stream())
     return host(out)
 
 
@@ -115,17 +156,39 @@ def bias_add(x, b, bf16=False):
     return host(out)
 
 
-def bias_add_grad(g, bf16=False):
+def bias_add_grad(g, bf16=False, offset=0):
+    """offset: elements between the gradient's allocation and the pointer passed."""
     L = lib()
     c = g.shape[-1]
     rows = g.size // max(c, 1)
-    dg = dev(g, bf16)
+    dg, pg = offset_copy(g, bf16, offset)
     out = empty((c,), tdt(bf16), fill=float("nan"))
     nb = L.b200_bias_add_grad_workspace_bytes(cdt(bf16), rows, c)
     w = ws(nb)
-    call(L.b200_bias_add_grad, cdt(bf16), dg.data_ptr(), out.data_ptr(), rows, c, w.data_ptr(), nb,
-         stream())
+    call(L.b200_bias_add_grad, cdt(bf16), pg, out.data_ptr(), rows, c, w.data_ptr(), nb, stream())
     return host(out)
+
+
+def relu_grad_bias_grad(g, f, bf16=False, offset=0, alias=False):
+    """b200_relu_grad_bias_grad on [rows, channels] = g.shape -> (backprops, bias_grad).
+    offset: elements between each allocation and the pointer passed; alias: backprops written over
+    the gradients buffer."""
+    L = lib()
+    c = g.shape[-1]
+    rows = g.size // max(c, 1)
+    dg, pg = offset_copy(g, bf16, offset)
+    df, pf = offset_copy(f, bf16, offset)
+    if alias:
+        dbp, pbp = dg, pg
+    else:
+        dbp = empty((g.size + offset,), tdt(bf16), fill=float("nan"))
+        pbp = dbp.data_ptr() + offset * dbp.element_size()
+    out = empty((c,), tdt(bf16), fill=float("nan"))
+    nb = L.b200_relu_grad_bias_grad_workspace_bytes(cdt(bf16), rows, c)
+    w = ws(nb)
+    call(L.b200_relu_grad_bias_grad, cdt(bf16), pg, pf, pbp, out.data_ptr(), rows, c, w.data_ptr(),
+         nb, stream())
+    return host(dbp)[offset:].reshape(g.shape), host(out)
 
 
 def bias_add_nchw(x, b, bf16=False):
@@ -182,6 +245,39 @@ def softmax_xent(logits, labels, bf16=False):
     call(lib().b200_softmax_xent, cdt(bf16), dl.data_ptr(), dlab.data_ptr(), loss.data_ptr(),
          bp.data_ptr(), logits.shape[0], logits.shape[1], stream())
     return host(loss), host(bp)
+
+
+def softmax_xent_scaled(logits, labels, scale, bf16=False, offset=0):
+    """b200_softmax_xent_scaled; scale: a float (uploaded as a device scalar) or None (NULL).
+    offset: elements between the logits allocation and the pointer passed."""
+    rows, cols = logits.shape
+    dl, pl = offset_copy(logits, bf16, offset)
+    dlab = dev(labels, bf16)
+    dsc = dev(np.array([scale], np.float32)) if scale is not None else None
+    loss = empty((rows,), tdt(bf16), fill=float("nan"))
+    bp = empty((rows, cols), tdt(bf16), fill=float("nan"))
+    call(lib().b200_softmax_xent_scaled, cdt(bf16), pl, dlab.data_ptr(), loss.data_ptr(),
+         bp.data_ptr(), rows, cols, dsc.data_ptr() if dsc is not None else None, stream())
+    return host(loss), host(bp)
+
+
+def mul_scalar(x, y, bf16=False):
+    """b200_mul with y a device scalar broadcast over x."""
+    dx, dy = dev(x, bf16), dev(np.array([y], np.float32), bf16)
+    out = empty(x.shape, tdt(bf16), fill=float("nan"))
+    call(lib().b200_mul, cdt(bf16), dx.data_ptr(), dy.data_ptr(), out.data_ptr(), x.size, 1,
+         stream())
+    return host(out)
+
+
+def reduce(x, scale=1.0, bf16=False):
+    """b200_reduce over axis 1 of x viewed as [outer, reduce, inner] -> [outer, inner]."""
+    outer, red, inner = x.shape
+    dx = dev(x, bf16) if x.size else ws(16)
+    out = empty((outer, inner), tdt(bf16), fill=float("nan"))
+    call(lib().b200_reduce, cdt(bf16), dx.data_ptr(), out.data_ptr(), outer, red, inner, scale,
+         stream())
+    return host(out)
 
 
 def max_pool(x, ksize, strides, padding, oracle, bf16=False):
@@ -285,6 +381,21 @@ def conv2d(x, f, strides, padding, oracle, bf16=False):
     w = ws(nb)
     call(L.b200_conv2d, cdt(bf16), dx.data_ptr(), df.data_ptr(), out.data_ptr(), ctypes.byref(g),
          w.data_ptr(), nb, stream())
+    return host(out)
+
+
+def fused_conv2d(x, f, bias, relu, strides, padding, oracle, bf16=False):
+    """b200_fused_conv2d (bias may be None) with the workspace b200_conv2d would get."""
+    L = lib()
+    g = _geom(oracle, x.shape, f.shape, strides, padding)
+    dx, df = dev(x, bf16), dev(f, bf16)
+    dbias = dev(bias, bf16) if bias is not None else None
+    out = empty((g.batch, g.out_h, g.out_w, g.out_c), tdt(bf16), fill=float("nan"))
+    nb = L.b200_conv2d_workspace_bytes(cdt(bf16), ctypes.byref(g), 0)
+    w = ws(nb)
+    call(L.b200_fused_conv2d, cdt(bf16), dx.data_ptr(), df.data_ptr(),
+         dbias.data_ptr() if dbias is not None else None, int(relu), out.data_ptr(),
+         ctypes.byref(g), w.data_ptr(), nb, stream())
     return host(out)
 
 

@@ -585,6 +585,20 @@ def test_sum_and_mean_reductions(oracle, rng, bf16):
             np.testing.assert_allclose(g, ref, rtol=1e-2 if bf16 else 1e-5, atol=1e-2 if bf16 else 1e-5)
 
 
+def test_reduce_sum_middle_axis_with_more_than_65535_outer_rows(rng):
+    # [70000, 10, 3] reduced over axis 1 collapses to outer = 70000, inner = 3: more outer rows than
+    # one grid dimension holds
+    x = rng.uniform(-1, 1, (70000, 10, 3)).astype(np.float32)
+    tf.reset_default_graph()
+    xp = tf.placeholder(tf.float32, list(x.shape), "x")
+    y = tf.reduce_sum(xp, 1)
+    with client.Session(tf.get_default_graph()) as sess:
+        got = sess.run(y, {xp: x})
+    ref = x.astype(np.float64).sum(1)
+    assert got.shape == ref.shape
+    assert (np.abs(got - ref) <= 1e-5 * np.abs(x).astype(np.float64).sum(1)).all()
+
+
 def test_alternating_reduction_axes_are_rejected(rng):
     tf.reset_default_graph()
     xp = tf.placeholder(tf.float32, [3, 4, 5], "x")
