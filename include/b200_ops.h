@@ -159,6 +159,24 @@ B200_API int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void*
                                   int64_t n, int64_t k, int transpose_a, int transpose_b,
                                   const void* bias, int relu, const void* relu_grad_features,
                                   void* workspace, size_t workspace_bytes, void* stream);
+/* Two independent products with the arguments of b200_fused_matmul_ws each (one dtype), computed
+ * as two b200_fused_matmul_ws calls would compute them, bit for bit.  When both run on the tensor
+ * cores with the same tile config and one is K-major x K-major (dX = dY W^T: transpose_b) while
+ * the other is MN-major x MN-major (dW = X^T dY: transpose_a), they share one persistent launch:
+ * the second product's operand fill and main loop hide the first one's epilogue, and the CTA
+ * pairs one product would leave idle get work.  Otherwise they run one after the other.
+ * workspace (optional): b200_matmul_pair_workspace_bytes() bytes; product 0's split-K scratch
+ * (b200_matmul_workspace_bytes of its shape) sits at offset 0, product 1's at the next 256-byte
+ * boundary after it. */
+B200_API size_t b200_matmul_pair_workspace_bytes(int dtype, int64_t m0, int64_t n0, int64_t k0,
+                                                 int64_t m1, int64_t n1, int64_t k1);
+B200_API int b200_matmul_pair(int dtype, const void* a0, const void* b0, void* c0, int64_t m0,
+                              int64_t n0, int64_t k0, int transpose_a0, int transpose_b0,
+                              const void* bias0, int relu0, const void* relu_grad_features0,
+                              const void* a1, const void* b1, void* c1, int64_t m1, int64_t n1,
+                              int64_t k1, int transpose_a1, int transpose_b1, const void* bias1,
+                              int relu1, const void* relu_grad_features1, void* workspace,
+                              size_t workspace_bytes, void* stream);
 /* Replaces LaunchBatchMatMul<GPUDevice,Scalar>::Launch -> ThenBlasGemmBatchedWithScratch
  * (core/kernels/batch_matmul_op_impl.h:297-363).  x is [batch,m,k] (or [batch,k,m] when adj_x),
  * y is [batch,k,n] (or [batch,n,k] when adj_y); strided, no pointer arrays, no scratch. */

@@ -76,6 +76,12 @@ SIGNATURES = {
                                   c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "b200_fused_matmul_ws": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                                   c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "b200_matmul_pair_workspace_bytes": (c_size_t, [c_int, c_int64, c_int64, c_int64, c_int64,
+                                                    c_int64, c_int64]),
+    "b200_matmul_pair": (c_int, [c_int]
+                         + [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_int,
+                            c_void_p, c_int, c_void_p] * 2
+                         + [c_void_p, c_size_t, c_void_p]),
     "b200_batch_matmul": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                                   c_int64, c_int, c_int, c_void_p]),
     "b200_bias_add": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p]),

@@ -83,6 +83,11 @@ bool gemm_tcgen05_supported(const GemmArgs& g);
 // Can this convolution's patch operand be fetched by TMA im2col (channel / padding limits)?
 bool conv_a_supported(int dtype, const ConvAOperand& c);
 int gemm_tcgen05(const GemmArgs& g, cudaStream_t stream);
+// Two independent tensor-core GEMMs of one dtype (both gemm_tcgen05-eligible) in one persistent
+// launch when they share a tile config and their majorness pair is instantiated (one K-major x
+// K-major, one MN-major x MN-major: a dense layer's dX and dW); otherwise gemm_tcgen05(a) then
+// gemm_tcgen05(b).  Results are bit-identical to the two separate launches.
+int gemm_tcgen05_pair(const GemmArgs& a, const GemmArgs& b, cudaStream_t stream);
 int gemm_simt(const GemmArgs& g, cudaStream_t stream);
 // Precision-aware front door used by matmul / batch_matmul / conv.
 int gemm_dispatch(const GemmArgs& g, cudaStream_t stream);

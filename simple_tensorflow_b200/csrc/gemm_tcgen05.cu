@@ -25,6 +25,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 namespace b200 {
 
@@ -113,6 +114,22 @@ __device__ __forceinline__ void trace_mark(const GemmShape& s, int slot, bool la
 
 __device__ __forceinline__ bool partial_out_tile(const GemmShape& s) { return s.splits > 1; }
 
+// One GEMM of a launch: operand maps, output (or partial-buffer) store map, ReluGrad-feature map.
+template <typename TOut>
+struct GemmProblem {
+  CUtensorMap tmapA, tmapB, tmapC, tmapF;
+  TOut* C;
+  GemmShape s;
+};
+// kNP = 1: one GEMM.  kNP = 2: two independent GEMMs with the same tile config in one persistent
+// launch (a dense layer's dX and dW); the flat work list holds the `first_work` items of problem
+// `first`, then those of the other one.
+template <typename TOut, int kNP>
+struct GemmParams {
+  GemmProblem<TOut> p[kNP];
+  int first, first_work;
+};
+
 __device__ __forceinline__ void store_row32(float* dst, const uint32_t (&v)[32], int ncols,
                                             bool vec_ok) {
   if (vec_ok && ncols == 32) {
@@ -194,17 +211,18 @@ __device__ __forceinline__ void store_out1(__nv_bfloat16* dst, float a) {
 }
 
 // TIn: operand element type (float -> tf32 MMA, bf16 -> f16-kind MMA); TOut: stored type.
-template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas>
+// (kAMN, kBMN): operand majorness of problem 0; (kAMN1, kBMN1): that of problem 1 when kNP = 2.
+// Each problem's majorness stays a compile-time constant: every role selects the problem of a
+// work item with one warp-uniform branch and runs a loop instantiated for it.
+template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas, int kNP = 1,
+          bool kAMN1 = false, bool kBMN1 = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
-gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
-                    const __grid_constant__ CUtensorMap tmapB,
-                    const __grid_constant__ CUtensorMap tmapC,
-                    const __grid_constant__ CUtensorMap tmapF, TOut* __restrict__ C,
-                    GemmShape s) {
+gemm_tcgen05_kernel(const __grid_constant__ GemmParams<TOut, kNP> P) {
+  static_assert(kNP == 1 || kNP == 2, "one or two problems");
   pdl_launch_dependents();
   if (threadIdx.x == 0) {
-    trace_mark(s, 0);
-    trace_mark(s, 9, true);
+    trace_mark(P.p[0].s, 0);
+    trace_mark(P.p[0].s, 9, true);
   }
   using Tr = GemmTraits<TIn>;
   constexpr int BK = Tr::kBK;
@@ -216,7 +234,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
   constexpr int kChunk = kSwizzleBytes / sizeof(TIn);  // MN elements per 128-B swizzle row
   constexpr int kTmemCols = 2 * BN;                    // double-buffered fp32 accumulator
   static_assert(kTmemCols <= 512 && (kTmemCols & (kTmemCols - 1)) == 0, "TMEM cols");
-  constexpr uint32_t kIdesc = make_idesc(Tr::kFormat, kAMN, kBMN, kTileM, BN);
 
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -241,19 +258,44 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
   const int unit = blockIdx.x / kCtas;        // tile scheduler unit: a CTA or a CTA pair
   const int num_units = gridDim.x / kCtas;
 
-  const int tiles_m = (s.M + kTileM - 1) / kTileM;
-  const int tiles_n = (s.N + BN - 1) / BN;
-  const int tiles_per_batch = tiles_m * tiles_n;
-  const int num_tiles = tiles_per_batch * s.batch;
-  const int num_kb = (s.K + BK - 1) / BK;
-  // Work item = (split, tile): consecutive units take different tiles of the same K split.
-  const int num_work = num_tiles * s.splits;
+  // Work item = (problem, split, tile): consecutive units take different tiles of the same K split.
+  auto tiles_of = [](const GemmShape& s) {
+    return ((s.M + kTileM - 1) / kTileM) * ((s.N + BN - 1) / BN) * s.batch;
+  };
+  int num_work = tiles_of(P.p[0].s) * P.p[0].s.splits;
+  if constexpr (kNP == 2) num_work += tiles_of(P.p[1].s) * P.p[1].s.splits;
+  // body(problem, item index within the problem, kAMN tag, kBMN tag) for flat work item `work`
+  auto with_item = [&](int work, auto&& body) {
+    if constexpr (kNP == 1) {
+      body(P.p[0], work, std::bool_constant<kAMN>{}, std::bool_constant<kBMN>{});
+    } else {
+      const bool in_first = work < P.first_work;
+      const int w = in_first ? work : work - P.first_work;
+      if (in_first == (P.first == 0))
+        body(P.p[0], w, std::bool_constant<kAMN>{}, std::bool_constant<kBMN>{});
+      else
+        body(P.p[1], w, std::bool_constant<kAMN1>{}, std::bool_constant<kBMN1>{});
+    }
+  };
+  // the same for a body that does not depend on the operand majorness: one instance, problem
+  // selected by a runtime index
+  auto with_problem = [&](int work, auto&& body) {
+    if constexpr (kNP == 1) {
+      body(P.p[0], work);
+    } else {
+      const bool in_first = work < P.first_work;
+      body(P.p[in_first ? P.first : 1 - P.first], in_first ? work : work - P.first_work);
+    }
+  };
 
   if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmapA);
-    tma_prefetch_desc(&tmapB);
-    if (s.tma_store) tma_prefetch_desc(&tmapC);
-    if (s.feat_tma) tma_prefetch_desc(&tmapF);
+#pragma unroll
+    for (int i = 0; i < kNP; ++i) {
+      tma_prefetch_desc(&P.p[i].tmapA);
+      tma_prefetch_desc(&P.p[i].tmapB);
+      if (P.p[i].s.tma_store) tma_prefetch_desc(&P.p[i].tmapC);
+      if (P.p[i].s.feat_tma) tma_prefetch_desc(&P.p[i].tmapF);
+    }
   }
   if (warp == 1) {
     if (lane == 0) {
@@ -283,17 +325,24 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);  // warp-uniform value
   // Everything above overlapped the previous kernel's tail (programmatic dependent launch);
   // from here on this grid reads and writes global memory.
-  if (threadIdx.x == 0) trace_mark(s, 1);
+  if (threadIdx.x == 0) trace_mark(P.p[0].s, 1);
   pdl_wait();
-  if (threadIdx.x == 0) trace_mark(s, 2);
+  if (threadIdx.x == 0) trace_mark(P.p[0].s, 2);
 
   if (warp == 0) {
     // ===================== TMA producer (one per CTA) =====================
     if (lane == 0) {
       uint32_t stage = 0, phase = 0;
-      for (int work = unit; work < num_work; work += num_units) {
-        const int split = work / num_tiles;
-        const int tile = work - split * num_tiles;
+      for (int work = unit; work < num_work; work += num_units)
+        with_item(work, [&](const GemmProblem<TOut>& pr, int item, auto amn, auto bmn) {
+        constexpr bool kA = decltype(amn)::value, kB = decltype(bmn)::value;
+        const GemmShape& s = pr.s;
+        const int tiles_m = (s.M + kTileM - 1) / kTileM;
+        const int tiles_per_batch = tiles_m * ((s.N + BN - 1) / BN);
+        const int num_tiles = tiles_per_batch * s.batch;
+        const int num_kb = (s.K + BK - 1) / BK;
+        const int split = item / num_tiles;
+        const int tile = item - split * num_tiles;
         const int b = tile / tiles_per_batch;
         const int t = tile - b * tiles_per_batch;
         const int m0 = (t % tiles_m) * kTileM + (int)cta_rank * kBM;
@@ -311,7 +360,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
           }
           int k0 = kb * BK;
           int cv_c0 = 0, cv_r = 0, cv_s = 0;
-          if (s.conv_a && !kAMN) {  // kb -> (tap, channel block); B rows follow HWIO: (tap * C + c0)
+          if (s.conv_a && !kA) {  // kb -> (tap, channel block); B rows follow HWIO: (tap * C + c0)
             const int tap = kb / s.cv_cblocks;
             cv_c0 = (kb - tap * s.cv_cblocks) * BK;
             cv_r = tap / s.cv_S;
@@ -334,7 +383,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
             else
               tma_load_4d(dst, map, &full_bar[stage], 0, k0, mn0 / kChunk, b);
           };
-          if (!kAMN && s.conv_a) {
+          if (!kA && s.conv_a) {
             // first output pixel of this CTA's 128-row slab -> input-space base coordinates
             const int ow = m0 % s.cv_OW;
             const int t2 = m0 / s.cv_OW;
@@ -342,13 +391,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
             const int img = t2 / s.cv_OH;
             const int bw = ow * s.cv_sw - s.cv_pl, bh = oh * s.cv_sh - s.cv_pt;
             if (kCtas == 2)
-              tma_load_im2col_4d_2cta(a_dst, &tmapA, &full_bar[stage], cv_c0, bw, bh, img,
+              tma_load_im2col_4d_2cta(a_dst, &pr.tmapA, &full_bar[stage], cv_c0, bw, bh, img,
                                       (uint16_t)cv_s, (uint16_t)cv_r);
             else
-              tma_load_im2col_4d(a_dst, &tmapA, &full_bar[stage], cv_c0, bw, bh, img,
+              tma_load_im2col_4d(a_dst, &pr.tmapA, &full_bar[stage], cv_c0, bw, bh, img,
                                  (uint16_t)cv_s, (uint16_t)cv_r);
-          } else if (!kAMN) {
-            load(a_dst, &tmapA, k0, m0);
+          } else if (!kA) {
+            load(a_dst, &pr.tmapA, k0, m0);
           } else if (s.conv_a) {
             // Filter gradient: GEMM-K runs over output pixels, GEMM-M over (tap, channel).  Each
             // 128-byte chunk of M is one (tap, channel block): an im2col box of BK pixels x chunk
@@ -367,34 +416,34 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
               if (tap >= s.cv_taps) tap = s.cv_taps - 1;  // rows beyond R*S*C are never stored
               const int fr = tap / s.cv_S, fs = tap - fr * s.cv_S;
               if (kCtas == 2)
-                tma_load_im2col_4d_2cta(a_dst + c * (BK * kSwizzleBytes), &tmapA, &full_bar[stage],
+                tma_load_im2col_4d_2cta(a_dst + c * (BK * kSwizzleBytes), &pr.tmapA, &full_bar[stage],
                                         c0, bw, bh, img, (uint16_t)fs, (uint16_t)fr);
               else
-                tma_load_im2col_4d(a_dst + c * (BK * kSwizzleBytes), &tmapA, &full_bar[stage], c0,
+                tma_load_im2col_4d(a_dst + c * (BK * kSwizzleBytes), &pr.tmapA, &full_bar[stage], c0,
                                    bw, bh, img, (uint16_t)fs, (uint16_t)fr);
             }
           } else if (s.a_map4d) {
-            load4(a_dst, &tmapA, m0);
+            load4(a_dst, &pr.tmapA, m0);
           } else {
 #pragma unroll
             for (int c = 0; c < kBM / kChunk; ++c)
-              load(a_dst + c * (BK * kSwizzleBytes), &tmapA, m0 + c * kChunk, k0);
+              load(a_dst + c * (BK * kSwizzleBytes), &pr.tmapA, m0 + c * kChunk, k0);
           }
-          if (!kBMN) {
-            load(b_dst, &tmapB, k0, n0);
+          if (!kB) {
+            load(b_dst, &pr.tmapB, k0, n0);
           } else if (s.b_map4d) {
-            load4(b_dst, &tmapB, n0);
+            load4(b_dst, &pr.tmapB, n0);
           } else {
 #pragma unroll
             for (int c = 0; c < kBNLocal / kChunk; ++c)
-              load(b_dst + c * (BK * kSwizzleBytes), &tmapB, n0 + c * kChunk, k0);
+              load(b_dst + c * (BK * kSwizzleBytes), &pr.tmapB, n0 + c * kChunk, k0);
           }
           if (++stage == kStages) {
             stage = 0;
             phase ^= 1;
           }
         }
-      }
+      });
     }
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA only when paired) =====================
@@ -405,21 +454,27 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
     if (leader) {
       uint32_t stage = 0, phase = 0;
       uint32_t acc = 0, acc_phase = 0;
-      // MN-major tf32 must use the 32-byte-atom 128B swizzle: 4-row (512 B) K groups.
-      constexpr bool kMn32 = sizeof(TIn) == 4;
-      // descriptors of stage 0, k step 0: later ones differ only in the start-address field
-      const uint64_t adesc0 = kAMN ? make_smem_desc_sw128(smem_u32(smA), BK * kSwizzleBytes,
+      for (int work = unit; work < num_work; work += num_units)
+        with_item(work, [&](const GemmProblem<TOut>& pr, int item, auto amn, auto bmn) {
+        constexpr bool kA = decltype(amn)::value, kB = decltype(bmn)::value;
+        constexpr uint32_t kIdesc = make_idesc(Tr::kFormat, kA, kB, kTileM, BN);
+        // MN-major tf32 must use the 32-byte-atom 128B swizzle: 4-row (512 B) K groups.
+        constexpr bool kMn32 = sizeof(TIn) == 4;
+        // descriptors of stage 0, k step 0: later ones differ only in the start-address field
+        const uint64_t adesc0 = kA ? make_smem_desc_sw128(smem_u32(smA), BK * kSwizzleBytes,
                                                           kMn32 ? 512 : 1024, kMn32 ? 1 : 2)
                                    : make_smem_desc_sw128(smem_u32(smA), 16, 1024);
-      const uint64_t bdesc0 = kBMN ? make_smem_desc_sw128(smem_u32(smB), BK * kSwizzleBytes,
+        const uint64_t bdesc0 = kB ? make_smem_desc_sw128(smem_u32(smB), BK * kSwizzleBytes,
                                                           kMn32 ? 512 : 1024, kMn32 ? 1 : 2)
                                    : make_smem_desc_sw128(smem_u32(smB), 16, 1024);
-      const uint32_t a_hi = (uint32_t)(adesc0 >> 32), b_hi = (uint32_t)(bdesc0 >> 32);
-      // K-major: advance 32 B inside the 128-B swizzle row; MN-major: advance kUmmaK rows.
-      constexpr uint32_t kAStep = (kAMN ? Tr::kUmmaK * kSwizzleBytes : Tr::kUmmaK * (int)sizeof(TIn)) >> 4;
-      constexpr uint32_t kBStep = (kBMN ? Tr::kUmmaK * kSwizzleBytes : Tr::kUmmaK * (int)sizeof(TIn)) >> 4;
-      for (int work = unit; work < num_work; work += num_units) {
-        const int split = work / num_tiles;
+        const uint32_t a_hi = (uint32_t)(adesc0 >> 32), b_hi = (uint32_t)(bdesc0 >> 32);
+        // K-major: advance 32 B inside the 128-B swizzle row; MN-major: advance kUmmaK rows.
+        constexpr uint32_t kAStep = (kA ? Tr::kUmmaK * kSwizzleBytes : Tr::kUmmaK * (int)sizeof(TIn)) >> 4;
+        constexpr uint32_t kBStep = (kB ? Tr::kUmmaK * kSwizzleBytes : Tr::kUmmaK * (int)sizeof(TIn)) >> 4;
+        const GemmShape& s = pr.s;
+        const int num_tiles = tiles_of(s);
+        const int num_kb = (s.K + BK - 1) / BK;
+        const int split = item / num_tiles;
         const int kb0 = split * s.kb_per_split;
         const int kb1 = min(kb0 + s.kb_per_split, num_kb);
         mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
@@ -469,7 +524,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
           acc = 0;
           acc_phase ^= 1;
         }
-      }
+      });
     }
   } else {
     // ===================== epilogue warps =====================
@@ -485,28 +540,36 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
     uint8_t* my_feat = smFeat + quad * kFeatBufs * kEpiBufBytes;
     uint64_t* my_fbar = feat_bar + quad * kFeatBufs;
     uint32_t feat_issued = 0, feat_used = 0;  // running chunk counters (buffer = n % kFeatBufs)
-    const bool feat_on = s.relu_grad_features != nullptr && s.feat_tma && s.splits == 1;
-    // ReluGrad features do not depend on the MMA: fetch them (coalesced, via TMA) ahead of use.
-    auto issue_feat = [&](int col, int row0f, int bidx) {
-      if (lane == 0) {
-        uint64_t* fb = &my_fbar[feat_issued % kFeatBufs];
-        mbar_expect_tx(fb, kEpiBufBytes);
-        tma_load_3d(my_feat + (feat_issued % kFeatBufs) * kEpiBufBytes, &tmapF, fb, col, row0f,
-                    bidx);
-      }
-      ++feat_issued;
-    };
-    const bool vec_ok = (s.ldc % (16 / (int)sizeof(TOut)) == 0) &&
-                        (s.strideC % (16 / (int)sizeof(TOut)) == 0) &&
-                        ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
-    for (int work = unit; work < num_work; work += num_units) {
-      const int split = work / num_tiles;
-      const int tile = work - split * num_tiles;
+    for (int work = unit; work < num_work; work += num_units)
+      with_problem(work, [&](const GemmProblem<TOut>& pr, int item) {
+      const GemmShape& s = pr.s;
+      TOut* __restrict__ C = pr.C;
+      const int tiles_m = (s.M + kTileM - 1) / kTileM;
+      const int tiles_per_batch = tiles_m * ((s.N + BN - 1) / BN);
+      const int num_tiles = tiles_per_batch * s.batch;
+      const bool feat_on = s.relu_grad_features != nullptr && s.feat_tma && s.splits == 1;
+      // ReluGrad features do not depend on the MMA: fetch them (coalesced, via TMA) ahead of use.
+      auto issue_feat = [&](int col, int row0f, int bidx) {
+        if (lane == 0) {
+          uint64_t* fb = &my_fbar[feat_issued % kFeatBufs];
+          mbar_expect_tx(fb, kEpiBufBytes);
+          tma_load_3d(my_feat + (feat_issued % kFeatBufs) * kEpiBufBytes, &pr.tmapF, fb, col,
+                      row0f, bidx);
+        }
+        ++feat_issued;
+      };
+      const bool vec_ok = (s.ldc % (16 / (int)sizeof(TOut)) == 0) &&
+                          (s.strideC % (16 / (int)sizeof(TOut)) == 0) &&
+                          ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
+      const int split = item / num_tiles;
+      const int tile = item - split * num_tiles;
       const int b = tile / tiles_per_batch;
       const int t = tile - b * tiles_per_batch;
       const int m0 = (t % tiles_m) * kTileM + (int)cta_rank * kBM;
       const int n0 = (t / tiles_m) * BN;
       const int row0 = m0 + quad * 32;
+      // the other problem's last item may have staged its bias here with generic stores
+      if (kNP == 2 && feat_on && lane == 0) fence_proxy_async_smem();
       if (feat_on) {  // the first kFeatBufs chunks of this tile, while the MMAs are still running
 #pragma unroll
         for (int pc = 0; pc < kFeatBufs; ++pc)
@@ -668,7 +731,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
-            tma_store_3d(&tmapC, buf, col, row0, partial_out ? split * s.batch + b : b);
+            tma_store_3d(&pr.tmapC, buf, col, row0, partial_out ? split * s.batch + b : b);
             tma_store_commit();
           }
           ++stores_in_flight;
@@ -800,10 +863,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
           }
         }
       }
-    }
-    if (warp == 2 && lane == 0) trace_mark(s, 6);
-    if (s.tma_store && lane == 0) tma_store_wait<0>();  // global writes done before exit
-    if (warp == 2 && lane == 0) trace_mark(s, 7);
+    });
+    if (warp == 2 && lane == 0) trace_mark(P.p[0].s, 6);
+    if ((P.p[0].s.tma_store || P.p[kNP - 1].s.tma_store) && lane == 0)
+      tma_store_wait<0>();  // global writes done before exit
+    if (warp == 2 && lane == 0) trace_mark(P.p[0].s, 7);
   }
 
   tc_fence_before();
@@ -819,8 +883,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmapA,
       tmem_dealloc<kTmemCols>(tmem_base);
   }
   if (threadIdx.x == 0) {
-    trace_mark(s, 8);
-    trace_mark(s, 10, true);
+    trace_mark(P.p[0].s, 8);
+    trace_mark(P.p[0].s, 10, true);
   }
 }
 
@@ -1022,13 +1086,16 @@ static bool encode_store_map(CUtensorMap* map, CUtensorMapDataType dt, size_t es
                                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// Tensor maps and shape of one GEMM for a launch with BN x kCtas tiles.  The split-K plan is the
+// one the GEMM's own launch uses, whether it runs alone or as one problem of a pair launch.
 template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas>
-static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
+static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* tiles_out) {
   using Tr = GemmTraits<TIn>;
   constexpr int kChunk = kSwizzleBytes / sizeof(TIn);
   constexpr int kTileM = kBM * kCtas;
   constexpr int kBNLocal = BN / kCtas;
-  CUtensorMap ma, mb;
+  CUtensorMap& ma = pr.tmapA;
+  CUtensorMap& mb = pr.tmapB;
   int rc;
   // A: logical [M,K]; stored [M,K] (K-major) or [K,M] (MN-major).  Box = one CTA's 128 rows.
   static const bool no_map4d = getenv("B200TF_GEMM_NO_MAP4D") != nullptr;
@@ -1062,19 +1129,9 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
                             g.strideB, kChunk, Tr::kBK, true);
   if (rc) return rc;
 
-  auto kern = gemm_tcgen05_kernel<TIn, TOut, kAMN, kBMN, BN, kCtas>;
-  static bool attr_set = false;  // per template instantiation
-  constexpr size_t smem = gemm_smem_bytes<BN, kCtas>();
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
-    if (e != cudaSuccess) {
-      set_last_error("cudaFuncSetAttribute(smem=%zu): %s", smem, cudaGetErrorString(e));
-      return B200_INTERNAL;
-    }
-    attr_set = true;
-  }
-  GemmShape s;
+  GemmShape& s = pr.s;
+  memset(&s, 0, sizeof(s));
+  pr.C = static_cast<TOut*>(g.c);
   s.M = (int)g.M;
   s.N = (int)g.N;
   s.K = (int)g.K;
@@ -1082,6 +1139,7 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
   s.ldc = (int)g.ldc;
   s.strideC = g.strideC;
   const long long tiles = ((g.M + kTileM - 1) / kTileM) * ((g.N + BN - 1) / BN) * g.batch;
+  *tiles_out = tiles;
   const int units = sm_count() / kCtas;  // schedulable CTAs or CTA pairs
   // split-K when the output tiles alone cannot fill the SMs and scratch was provided
   const int num_kb = (int)((g.K + Tr::kBK - 1) / Tr::kBK);
@@ -1113,7 +1171,7 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
   s.relu = g.relu ? 1 : 0;
   s.relu_grad_features = g.relu_grad_features;
   s.ld_features = (int)g.ld_features;
-  CUtensorMap mc;
+  CUtensorMap& mc = pr.tmapC;
   memset(&mc, 0, sizeof(mc));
   static const bool no_tma_store = getenv("B200TF_GEMM_DIRECT_STORE") != nullptr;
   if (no_tma_store)
@@ -1125,7 +1183,7 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
     s.tma_store = encode_store_map(&mc, sizeof(TOut) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
                                                           : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16,
                                    sizeof(TOut), g.c, g.M, g.N, g.ldc, g.batch, g.strideC);
-  CUtensorMap mf;
+  CUtensorMap& mf = pr.tmapF;
   memset(&mf, 0, sizeof(mf));
   s.feat_tma = 0;
   if (g.relu_grad_features && splits == 1)
@@ -1134,9 +1192,146 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
                                   sizeof(TOut), const_cast<void*>(g.relu_grad_features), g.M, g.N,
                                   g.ld_features, 1, g.M * g.ld_features);
   s.bias_vec = g.bias && (reinterpret_cast<uintptr_t>(g.bias) & 15) == 0;
+  s.trace = nullptr;
+  s.tickets = nullptr;
+  return B200_OK;
+}
+
+// One persistent launch of `kern` over grid_units CTAs (pairs): cluster and PDL attributes,
+// the one-time shared-memory opt-in, and the B200TF_KERNEL_TIMES bracket.
+template <typename TOut, int kNP>
+static int launch_persistent(void (*kern)(GemmParams<TOut, kNP>), bool& attr_set,
+                             const GemmParams<TOut, kNP>& P, int grid_units, int ctas, size_t smem,
+                             bool pdl, cudaStream_t stream) {
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) {
+      set_last_error("cudaFuncSetAttribute(smem=%zu): %s", smem, cudaGetErrorString(e));
+      return B200_INTERNAL;
+    }
+    attr_set = true;
+  }
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid_units * ctas);
+  cfg.blockDim = dim3(kGemmThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[2];
+  int na = 0;
+  if (ctas > 1) {
+    attr[na].id = cudaLaunchAttributeClusterDimension;
+    attr[na].val.clusterDim.x = ctas;
+    attr[na].val.clusterDim.y = 1;
+    attr[na].val.clusterDim.z = 1;
+    ++na;
+  }
+  if (pdl) {  // prologue overlaps the predecessor's tail; the kernel pdl_wait()s before global I/O
+    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
+  }
+  cfg.attrs = attr;
+  cfg.numAttrs = na;
+  void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, P);
+  if (ktok) kernel_times_end(ktok, stream, reinterpret_cast<const void*>(kern));
+  if (e != cudaSuccess) {
+    set_last_error("gemm_tcgen05 launch: %s", cudaGetErrorString(e));
+    cudaGetLastError();
+    return B200_INTERNAL;
+  }
+  return B200_OK;
+}
+
+// Ordered reduction of a split GEMM's fp32 partials into C (+ its bias / relu tail).
+template <typename TOut>
+static int launch_splitk_reduce(const GemmArgs& g, const GemmShape& s, bool pdl, bool prof,
+                                cudaStream_t stream) {
+  const int splits = s.splits;
+  const long long groups = g.batch * g.M * ((g.N + 3) / 4);
+  long long rblocks = (groups + 255) / 256;
+  if (rblocks > 8LL * sm_count()) rblocks = 8LL * sm_count();
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)rblocks);
+  cfg.blockDim = dim3(256);
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = pdl && !prof ? 1 : 0;
+  static const bool generic_only = getenv("B200TF_SPLITK_REDUCE_GENERIC") != nullptr;
+  const bool flat = !generic_only && (s.N & 3) == 0 && s.ldc == s.N &&
+                    (g.batch == 1 || (long long)s.strideC == (long long)s.M * s.N) &&
+                    splits >= 2 && splits <= 16 &&
+                    (reinterpret_cast<uintptr_t>(s.partial) & 15) == 0 &&
+                    (reinterpret_cast<uintptr_t>(g.c) & 15) == 0;
+  cudaError_t e;
+  void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
+  if (ktok) cfg.numAttrs = 0;
+  if (flat) {
+    const long long total4 = g.batch * (long long)s.M * (s.N / 4);
+    const float4* p4 = reinterpret_cast<const float4*>(s.partial);
+    TOut* c = static_cast<TOut*>(g.c);
+    const TOut* bias = static_cast<const TOut*>(g.bias);
+    const int relu = g.relu ? 1 : 0, n4 = s.N / 4;
+    switch (splits) {
+#define B200_SPLITK_FLAT(S_)                                                                   \
+  case S_:                                                                                     \
+    e = cudaLaunchKernelEx(&cfg, splitk_reduce_flat_kernel<TOut, S_>, p4, c, total4, total4, \
+                           n4, bias, relu);                                                    \
+    break;
+      B200_SPLITK_FLAT(2)
+      B200_SPLITK_FLAT(3)
+      B200_SPLITK_FLAT(4)
+      B200_SPLITK_FLAT(5)
+      B200_SPLITK_FLAT(6)
+      B200_SPLITK_FLAT(7)
+      B200_SPLITK_FLAT(8)
+      B200_SPLITK_FLAT(9)
+      B200_SPLITK_FLAT(10)
+      B200_SPLITK_FLAT(11)
+      B200_SPLITK_FLAT(12)
+      B200_SPLITK_FLAT(13)
+      B200_SPLITK_FLAT(14)
+      B200_SPLITK_FLAT(15)
+      default:
+      B200_SPLITK_FLAT(16)
+#undef B200_SPLITK_FLAT
+    }
+  } else {
+    e = cudaLaunchKernelEx(&cfg, splitk_reduce_kernel<TOut>,
+                           static_cast<const float*>(s.partial), static_cast<TOut*>(g.c),
+                           splits, (long long)g.batch, s.M, s.N, s.ldc,
+                           (long long)s.strideC, static_cast<const TOut*>(g.bias),
+                           g.relu ? 1 : 0);
+  }
+  if (ktok)
+    kernel_times_end(ktok, stream,
+                     flat ? reinterpret_cast<const void*>(splitk_reduce_flat_kernel<TOut, 4>)
+                          : reinterpret_cast<const void*>(splitk_reduce_kernel<TOut>));
+  if (e != cudaSuccess) {
+    set_last_error("splitk_reduce launch: %s", cudaGetErrorString(e));
+    cudaGetLastError();
+    return B200_INTERNAL;
+  }
+  note_launch();
+  return B200_OK;
+}
+
+template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas>
+static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
+  GemmParams<TOut, 1> P;
+  memset(&P, 0, sizeof(P));
+  long long tiles = 0;
+  int rc = prepare_problem<TIn, TOut, kAMN, kBMN, BN, kCtas>(g, P.p[0], &tiles);
+  if (rc) return rc;
+  GemmShape& s = P.p[0].s;
+  const int splits = s.splits;
+  const int units = sm_count() / kCtas;
   static const bool trace_on = getenv("B200TF_GEMM_TRACE") != nullptr;
   static unsigned long long* trace_buf = nullptr;
-  s.trace = nullptr;
   if (trace_on) {
     if (trace_buf == nullptr) cudaMalloc(&trace_buf, 16 * sizeof(unsigned long long));
     if (trace_buf != nullptr) {
@@ -1153,7 +1348,6 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
   // splits): 26.7 us in-kernel vs 26.6 us with the separate ordered pass, step time unchanged --
   // the wait for the slowest split plus the L2 round trips of the reduction cost what the second
   // launch costs -- so the simpler two-kernel form stays the default (profiles/r02_notes.md).
-  s.tickets = nullptr;
   static const bool inkernel_reduce = getenv("B200TF_SPLITK_INKERNEL") != nullptr;
   if (splits > 1 && inkernel_reduce && !g.bias && work <= units && tiles <= kSplitKMaxTiles) {
     static unsigned int* ticket_base[64] = {nullptr};
@@ -1176,37 +1370,10 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
   const bool prof = profile_enabled();
   if (prof) profile_gemm_launch_begin(stream);
   const bool pdl = pdl_enabled();
-  {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid_units * kCtas);
-    cfg.blockDim = dim3(kGemmThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (kCtas > 1) {
-      attr[na].id = cudaLaunchAttributeClusterDimension;
-      attr[na].val.clusterDim.x = kCtas;
-      attr[na].val.clusterDim.y = 1;
-      attr[na].val.clusterDim.z = 1;
-      ++na;
-    }
-    if (pdl) {  // prologue overlaps the predecessor's tail; the kernel pdl_wait()s before global I/O
-      attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[na].val.programmaticStreamSerializationAllowed = 1;
-      ++na;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
-    void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, ma, mb, mc, mf, static_cast<TOut*>(g.c), s);
-    if (ktok) kernel_times_end(ktok, stream, reinterpret_cast<const void*>(kern));
-    if (e != cudaSuccess) {
-      set_last_error("gemm_tcgen05 launch: %s", cudaGetErrorString(e));
-      cudaGetLastError();
-      return B200_INTERNAL;
-    }
-  }
+  static bool attr_set = false;  // per template instantiation
+  rc = launch_persistent<TOut, 1>(gemm_tcgen05_kernel<TIn, TOut, kAMN, kBMN, BN, kCtas>, attr_set,
+                                  P, grid_units, kCtas, gemm_smem_bytes<BN, kCtas>(), pdl, stream);
+  if (rc) return rc;
   if (prof) profile_gemm_launch_end(stream, 2.0 * (double)g.M * (double)g.N * (double)g.K * g.batch);
   if (s.trace != nullptr) {  // debug: phase boundaries, ns since the first CTA entered the kernel
     unsigned long long t[16];
@@ -1222,76 +1389,51 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
   }
   note_launch();
   if (splits > 1 && s.tickets == nullptr) {
-    const long long groups = g.batch * g.M * ((g.N + 3) / 4);
-    long long rblocks = (groups + 255) / 256;
-    if (rblocks > 8LL * sm_count()) rblocks = 8LL * sm_count();
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)rblocks);
-    cfg.blockDim = dim3(256);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl && !prof ? 1 : 0;
-    static const bool generic_only = getenv("B200TF_SPLITK_REDUCE_GENERIC") != nullptr;
-    const bool flat = !generic_only && (s.N & 3) == 0 && s.ldc == s.N &&
-                      (g.batch == 1 || (long long)s.strideC == (long long)s.M * s.N) &&
-                      splits >= 2 && splits <= 16 &&
-                      (reinterpret_cast<uintptr_t>(s.partial) & 15) == 0 &&
-                      (reinterpret_cast<uintptr_t>(g.c) & 15) == 0;
-    cudaError_t e;
-    void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
-    if (ktok) cfg.numAttrs = 0;
-    if (flat) {
-      const long long total4 = g.batch * (long long)s.M * (s.N / 4);
-      const float4* p4 = reinterpret_cast<const float4*>(s.partial);
-      TOut* c = static_cast<TOut*>(g.c);
-      const TOut* bias = static_cast<const TOut*>(g.bias);
-      const int relu = g.relu ? 1 : 0, n4 = s.N / 4;
-      switch (splits) {
-#define B200_SPLITK_FLAT(S_)                                                                   \
-  case S_:                                                                                     \
-    e = cudaLaunchKernelEx(&cfg, splitk_reduce_flat_kernel<TOut, S_>, p4, c, total4, total4, \
-                           n4, bias, relu);                                                    \
-    break;
-        B200_SPLITK_FLAT(2)
-        B200_SPLITK_FLAT(3)
-        B200_SPLITK_FLAT(4)
-        B200_SPLITK_FLAT(5)
-        B200_SPLITK_FLAT(6)
-        B200_SPLITK_FLAT(7)
-        B200_SPLITK_FLAT(8)
-        B200_SPLITK_FLAT(9)
-        B200_SPLITK_FLAT(10)
-        B200_SPLITK_FLAT(11)
-        B200_SPLITK_FLAT(12)
-        B200_SPLITK_FLAT(13)
-        B200_SPLITK_FLAT(14)
-        B200_SPLITK_FLAT(15)
-        default:
-        B200_SPLITK_FLAT(16)
-#undef B200_SPLITK_FLAT
-      }
-    } else {
-      e = cudaLaunchKernelEx(&cfg, splitk_reduce_kernel<TOut>,
-                             static_cast<const float*>(s.partial), static_cast<TOut*>(g.c),
-                             splits, (long long)g.batch, s.M, s.N, s.ldc,
-                             (long long)s.strideC, static_cast<const TOut*>(g.bias),
-                             g.relu ? 1 : 0);
-    }
-    if (ktok)
-      kernel_times_end(ktok, stream,
-                       flat ? reinterpret_cast<const void*>(splitk_reduce_flat_kernel<TOut, 4>)
-                            : reinterpret_cast<const void*>(splitk_reduce_kernel<TOut>));
-    if (e != cudaSuccess) {
-      set_last_error("splitk_reduce launch: %s", cudaGetErrorString(e));
-      cudaGetLastError();
-      return B200_INTERNAL;
-    }
-    note_launch();
+    rc = launch_splitk_reduce<TOut>(g, s, pdl, prof, stream);
+    if (rc) return rc;
   }
   return check_launch("gemm_tcgen05");
+}
+
+// A dense layer's input gradient dX = dY * W^T (slot 0: both operands K-major) and weight gradient
+// dW = X^T * dY (slot 1: both MN-major) in one persistent launch of BN-wide pair tiles.  Each
+// problem keeps the split plan, tile order and fused tail of its own launch, so every output is
+// bit-identical to it; split problems keep their own reduction pass afterwards.  The problem
+// whose items are longer comes first in the work list, so that the short items fill the tail.
+template <typename TIn, typename TOut, int BN>
+static int launch_gemm_pair(const GemmArgs& g0, const GemmArgs& g1, cudaStream_t stream) {
+  constexpr int kCtas = 2;
+  GemmParams<TOut, 2> P;
+  memset(&P, 0, sizeof(P));
+  long long tiles0 = 0, tiles1 = 0;
+  int rc = prepare_problem<TIn, TOut, false, false, BN, kCtas>(g0, P.p[0], &tiles0);
+  if (rc) return rc;
+  rc = prepare_problem<TIn, TOut, true, true, BN, kCtas>(g1, P.p[1], &tiles1);
+  if (rc) return rc;
+  const long long work0 = tiles0 * P.p[0].s.splits, work1 = tiles1 * P.p[1].s.splits;
+  P.first = P.p[1].s.kb_per_split > P.p[0].s.kb_per_split ? 1 : 0;
+  P.first_work = (int)(P.first ? work1 : work0);
+  const int units = sm_count() / kCtas;
+  const long long work = work0 + work1;
+  const int grid_units = (int)(work < units ? work : units);
+  const bool prof = profile_enabled();
+  if (prof) profile_gemm_launch_begin(stream);
+  const bool pdl = pdl_enabled();
+  static bool attr_set = false;  // per template instantiation
+  rc = launch_persistent<TOut, 2>(
+      gemm_tcgen05_kernel<TIn, TOut, false, false, BN, kCtas, 2, true, true>, attr_set, P,
+      grid_units, kCtas, gemm_smem_bytes<BN, kCtas>(), pdl, stream);
+  if (rc) return rc;
+  if (prof)
+    profile_gemm_launch_end(stream, 2.0 * ((double)g0.M * (double)g0.N * (double)g0.K +
+                                           (double)g1.M * (double)g1.N * (double)g1.K));
+  note_launch();
+  for (int i = 0; i < 2; ++i)
+    if (P.p[i].s.splits > 1) {
+      rc = launch_splitk_reduce<TOut>(i ? g1 : g0, P.p[i].s, pdl, prof, stream);
+      if (rc) return rc;
+    }
+  return check_launch("gemm_tcgen05_pair");
 }
 
 template <typename TIn, typename TOut, int BN, int kCtas>
@@ -1391,6 +1533,29 @@ int gemm_tcgen05(const GemmArgs& g, cudaStream_t stream) {
     return dispatch_config<__nv_bfloat16, __nv_bfloat16>(g, c, stream);
   set_last_error("gemm_tcgen05: unsupported dtype %d", g.dtype);
   return B200_UNIMPLEMENTED;
+}
+
+int gemm_tcgen05_pair(const GemmArgs& a, const GemmArgs& b, cudaStream_t stream) {
+  auto majors = [](const GemmArgs& g, bool mn) { return g.a_mn_major == mn && g.b_mn_major == mn; };
+  // slot 0 takes the K-major x K-major product, slot 1 the MN-major x MN-major one
+  const bool a_first = majors(a, false) && majors(b, true);
+  const GemmArgs& g0 = a_first ? a : b;
+  const GemmArgs& g1 = a_first ? b : a;
+  const TileConfig c0 = choose_config(g0), c1 = choose_config(g1);
+  const bool paired = a.dtype == b.dtype && majors(g0, false) && majors(g1, true) &&
+                      a.batch == 1 && b.batch == 1 && !a.conv_a && !b.conv_a &&
+                      gemm_tcgen05_supported(a) && gemm_tcgen05_supported(b) && c0.ctas == 2 &&
+                      c1.ctas == 2 && c0.bn == c1.bn;
+  if (!paired) {
+    const int rc = gemm_tcgen05(a, stream);
+    return rc ? rc : gemm_tcgen05(b, stream);
+  }
+  if (g0.dtype == B200_DT_FLOAT)
+    return c0.bn == 256 ? launch_gemm_pair<float, float, 256>(g0, g1, stream)
+                        : launch_gemm_pair<float, float, 128>(g0, g1, stream);
+  return c0.bn == 256
+             ? launch_gemm_pair<__nv_bfloat16, __nv_bfloat16, 256>(g0, g1, stream)
+             : launch_gemm_pair<__nv_bfloat16, __nv_bfloat16, 128>(g0, g1, stream);
 }
 
 }  // namespace b200

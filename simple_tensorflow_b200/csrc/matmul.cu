@@ -473,14 +473,19 @@ int b200_fused_matmul(int dtype, const void* a, const void* b, void* c, int64_t 
                               relu_grad_features, nullptr, 0, stream);
 }
 
-int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n,
-                         int64_t k, int transpose_a, int transpose_b, const void* bias, int relu,
-                         const void* relu_grad_features, void* workspace, size_t workspace_bytes,
-                         void* stream) {
-  int rc = validate_gemm("b200_fused_matmul", dtype, a, b, c, m, n, k, 1);
+}  // extern "C"
+
+namespace b200 {
+
+// Arguments of one (optionally fused) 2-D product, as b200_fused_matmul_ws takes them.
+static int fused_matmul_args(const char* what, int dtype, const void* a, const void* b, void* c,
+                             int64_t m, int64_t n, int64_t k, int transpose_a, int transpose_b,
+                             const void* bias, int relu, const void* relu_grad_features,
+                             void* workspace, size_t workspace_bytes, GemmArgs* out) {
+  int rc = validate_gemm(what, dtype, a, b, c, m, n, k, 1);
   if (rc) return rc;
   if (relu && relu_grad_features) {
-    set_last_error("b200_fused_matmul: relu and relu_grad_features are mutually exclusive");
+    set_last_error("%s: relu and relu_grad_features are mutually exclusive", what);
     return B200_INVALID_ARGUMENT;
   }
   GemmArgs g{};
@@ -508,15 +513,71 @@ int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void* c, int64
     g.workspace = workspace;  // enables split-K; the bias / relu tail moves to the reduction pass
     g.workspace_bytes = workspace_bytes;
   }
-  if (use_tcgen05(g)) return gemm_tcgen05(g, as_stream(stream));
+  *out = g;
+  return B200_OK;
+}
+
+static int fused_matmul(const GemmArgs& g, cudaStream_t stream) {
+  if (use_tcgen05(g)) return gemm_tcgen05(g, stream);
   // CUDA-core shapes (TMA cannot address them, tiny, matrix-vector) and exact mode: GEMM, then the
   // element-wise tail as separate kernels.
-  rc = gemm_simt(g, as_stream(stream));
+  int rc = gemm_simt(g, stream);
   if (rc) return rc;
-  if (bias) rc = b200_bias_add(dtype, c, bias, c, m, n, stream);
-  if (!rc && relu) rc = b200_relu(dtype, c, c, m * n, stream);
-  if (!rc && relu_grad_features) rc = b200_relu_grad(dtype, c, relu_grad_features, c, m * n, stream);
+  void* c = g.c;
+  if (g.bias) rc = b200_bias_add(g.dtype, c, g.bias, c, g.M, g.N, stream);
+  if (!rc && g.relu) rc = b200_relu(g.dtype, c, c, g.M * g.N, stream);
+  if (!rc && g.relu_grad_features)
+    rc = b200_relu_grad(g.dtype, c, g.relu_grad_features, c, g.M * g.N, stream);
   return rc;
+}
+
+static size_t align256(size_t x) { return (x + 255) & ~static_cast<size_t>(255); }
+
+}  // namespace b200
+
+extern "C" {
+
+int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n,
+                         int64_t k, int transpose_a, int transpose_b, const void* bias, int relu,
+                         const void* relu_grad_features, void* workspace, size_t workspace_bytes,
+                         void* stream) {
+  GemmArgs g;
+  const int rc = fused_matmul_args("b200_fused_matmul", dtype, a, b, c, m, n, k, transpose_a,
+                                   transpose_b, bias, relu, relu_grad_features, workspace,
+                                   workspace_bytes, &g);
+  return rc ? rc : fused_matmul(g, as_stream(stream));
+}
+
+size_t b200_matmul_pair_workspace_bytes(int dtype, int64_t m0, int64_t n0, int64_t k0, int64_t m1,
+                                        int64_t n1, int64_t k1) {
+  const size_t ws1 = gemm_workspace_bytes(dtype, m1, n1, k1, 1);
+  return ws1 ? align256(gemm_workspace_bytes(dtype, m0, n0, k0, 1)) + ws1
+             : gemm_workspace_bytes(dtype, m0, n0, k0, 1);
+}
+
+int b200_matmul_pair(int dtype, const void* a0, const void* b0, void* c0, int64_t m0, int64_t n0,
+                     int64_t k0, int transpose_a0, int transpose_b0, const void* bias0, int relu0,
+                     const void* relu_grad_features0, const void* a1, const void* b1, void* c1,
+                     int64_t m1, int64_t n1, int64_t k1, int transpose_a1, int transpose_b1,
+                     const void* bias1, int relu1, const void* relu_grad_features1,
+                     void* workspace, size_t workspace_bytes, void* stream) {
+  // product 0's scratch at offset 0, product 1's at the next 256-byte boundary past it
+  const size_t ws0 = workspace ? gemm_workspace_bytes(dtype, m0, n0, k0, 1) : 0;
+  const size_t off1 = align256(ws0);
+  void* w1 = workspace_bytes > off1 ? static_cast<char*>(workspace) + off1 : nullptr;
+  GemmArgs g0, g1;
+  int rc = fused_matmul_args("b200_matmul_pair", dtype, a0, b0, c0, m0, n0, k0, transpose_a0,
+                             transpose_b0, bias0, relu0, relu_grad_features0, workspace,
+                             std::min(ws0, workspace_bytes), &g0);
+  if (rc) return rc;
+  rc = fused_matmul_args("b200_matmul_pair", dtype, a1, b1, c1, m1, n1, k1, transpose_a1,
+                         transpose_b1, bias1, relu1, relu_grad_features1, w1,
+                         w1 ? workspace_bytes - off1 : 0, &g1);
+  if (rc) return rc;
+  const cudaStream_t s = as_stream(stream);
+  if (use_tcgen05(g0) && use_tcgen05(g1)) return gemm_tcgen05_pair(g0, g1, s);
+  rc = fused_matmul(g0, s);
+  return rc ? rc : fused_matmul(g1, s);
 }
 
 int b200_batch_matmul(int dtype, const void* x, const void* y, void* out, int64_t batch, int64_t m,

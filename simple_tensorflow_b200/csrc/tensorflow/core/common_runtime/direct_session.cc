@@ -341,6 +341,7 @@ Status DirectSession::GetOrCreateExecutors(const std::vector<std::string>& feeds
   ek->node_first_entry = first_entry;
   if (getenv("B200TF_DISABLE_FUSION") == nullptr) {
     TF_RETURN_IF_ERROR(FuseMatMulChains(ek.get()));
+    TF_RETURN_IF_ERROR(FuseSiblingMatMuls(ek.get()));
     TF_RETURN_IF_ERROR(FuseReluGradBiasGrad(ek.get()));
     TF_RETURN_IF_ERROR(FusePoolGradReluGradBiasGrad(ek.get()));
     TF_RETURN_IF_ERROR(FuseXentScale(ek.get()));
@@ -765,6 +766,94 @@ Status DirectSession::FuseMatMulChains(ExecutorsAndKeys* ek) {
     if (last != j) next.dead = true;
     ek->order[last] = repl;
     ek->rewritten.push_back(std::move(fused));
+  }
+  std::vector<PlanNode> alive;
+  for (PlanNode& pn : ek->order)
+    if (!pn.dead) alive.push_back(std::move(pn));
+  ek->order.swap(alive);
+  return Status::OK();
+}
+
+// Two live MatMul / _FusedMatMul nodes of one dtype that read the same tensor and have no fed
+// input -- a dense layer's dX = dY W^T (+ ReluGrad) and dW = X^T dY -- run as one _MatMulPair:
+// one persistent GEMM launch in which the second product's operand fill and main loop hide the
+// first one's epilogue, and the CTA pairs one product would leave idle get work.  The pair takes
+// the earlier node's place, so it is formed only when every input of the later node is produced
+// before that place (which also means the later node does not depend on the earlier one) and no
+// node in between updates a buffer the later node reads.  Each output keeps its entry, so the
+// consumers, fetches and gradient arenas of both products are unchanged.
+Status DirectSession::FuseSiblingMatMuls(ExecutorsAndKeys* ek) {
+  auto candidate = [&](const PlanNode& pn) {
+    if (pn.dead || (pn.item->def.op != "MatMul" && pn.item->def.op != "_FusedMatMul")) return false;
+    const DataType dt = pn.item->kernel->input_type(0);
+    if (dt != DT_FLOAT && dt != DT_BFLOAT16) return false;
+    for (const InputSource& in : pn.inputs)
+      if (in.feed >= 0) return false;
+    return true;
+  };
+  std::vector<int> producer_pos(ek->num_entries, -1);
+  for (size_t p = 0; p < ek->order.size(); ++p)
+    for (int o = 0; o < ek->order[p].item->kernel->num_outputs(); ++o)
+      producer_pos[ek->order[p].out_entry(o)] = static_cast<int>(p);
+  auto entry_of = [&](const InputSource& in) { return entry_index_of(ek, in.id); };
+  for (size_t i = 0; i < ek->order.size(); ++i) {
+    if (!candidate(ek->order[i])) continue;
+    const PlanNode& first = ek->order[i];
+    const DataType dt = first.item->kernel->input_type(0);
+    for (size_t j = i + 1; j < ek->order.size(); ++j) {
+      const PlanNode& second = ek->order[j];
+      if (!candidate(second) || second.item->kernel->input_type(0) != dt) continue;
+      bool shared = false, ready = true;
+      for (int x = 0; x < 2; ++x)
+        for (int y = 0; y < 2; ++y)
+          shared = shared || entry_of(first.inputs[x]) == entry_of(second.inputs[y]);
+      for (const InputSource& in : second.inputs)
+        ready = ready && producer_pos[entry_of(in)] < static_cast<int>(i);
+      if (!shared || !ready) continue;
+      // a variable update or an in-place all-reduce of one of its inputs must stay before it
+      bool clobbered = false;
+      for (size_t k = i + 1; k < j && !clobbered; ++k) {
+        const PlanNode& mid = ek->order[k];
+        if (mid.dead) continue;
+        for (DataType t : mid.item->kernel->input_types())
+          clobbered = clobbered || static_cast<int>(t) >= 100;  // a ref input
+        if (mid.item->def.op.rfind("B200AllReduce", 0) == 0)
+          for (const InputSource& a : mid.inputs)
+            for (const InputSource& b : second.inputs)
+              clobbered = clobbered || (a.feed < 0 && entry_of(a) == entry_of(b));
+      }
+      if (clobbered) continue;
+      std::unique_ptr<NodeItem> fused(new NodeItem);
+      fused->def.name = second.item->def.name + "/_matmul_pair";
+      fused->def.op = "_MatMulPair";
+      fused->def.attr["T"] = AttrValue::Type(dt);
+      const PlanNode* parts[2] = {&first, &second};
+      PlanNode repl;
+      repl.node = -1;
+      repl.first_entry = first.first_entry;
+      for (int q = 0; q < 2; ++q) {
+        const NodeDef& d = parts[q]->item->def;
+        const std::string sfx = q == 0 ? "0" : "1";
+        std::vector<std::string> ops;
+        GetNodeAttr(d, "fused_ops", &ops);
+        fused->def.attr["transpose_a" + sfx] = d.attr.at("transpose_a");
+        fused->def.attr["transpose_b" + sfx] = d.attr.at("transpose_b");
+        fused->def.attr["fused_ops" + sfx] = AttrValue::ListS(ops);
+        fused->def.attr["num_args" + sfx] =
+            AttrValue::I(static_cast<int64>(parts[q]->inputs.size()) - 2);
+        for (size_t x = 0; x < parts[q]->inputs.size(); ++x) {
+          repl.inputs.push_back(parts[q]->inputs[x]);
+          fused->def.input.push_back(d.input[x]);
+        }
+        repl.output_entries.push_back(parts[q]->out_entry(0));
+      }
+      TF_RETURN_IF_ERROR(EnsureKernel(fused.get()));
+      repl.item = fused.get();
+      ek->order[j].dead = true;
+      ek->order[i] = std::move(repl);
+      ek->rewritten.push_back(std::move(fused));
+      break;
+    }
   }
   std::vector<PlanNode> alive;
   for (PlanNode& pn : ek->order)

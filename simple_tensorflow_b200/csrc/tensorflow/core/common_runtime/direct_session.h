@@ -154,6 +154,9 @@ class DirectSession : public Session {
   // GraphOptimizer-stage rewrite (direct_session.cc:1051 role): MatMul+BiasAdd(+Relu) and
   // MatMul+ReluGrad chains whose intermediates have a single consumer run as one _FusedMatMul.
   Status FuseMatMulChains(ExecutorsAndKeys* ek);
+  // A dense layer's dX and dW products (two MatMuls reading the same tensor, neither depending on
+  // the other) run as one _MatMulPair: one persistent GEMM launch for both.
+  Status FuseSiblingMatMuls(ExecutorsAndKeys* ek);
   // SoftmaxCrossEntropyWithLogits whose backprop output only feeds Mul(backprop, scalar Const)
   // (the gradient of a mean loss, nn_grad.py:323-333 + math_grad.py _MeanGrad) runs as one
   // _ScaledSoftmaxCrossEntropyWithLogits: same fp32 roundings, one pass less over [batch, classes].

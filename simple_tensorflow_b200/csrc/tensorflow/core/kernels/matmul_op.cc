@@ -197,13 +197,142 @@ class FusedMatMulOp : public OpKernel {
   Mode mode_ = kBias;
 };
 
+// _MatMulPair: two independent products (a dense layer's dX and dW), each checked and allocated
+// as its own MatMul / _FusedMatMul would be, computed by one b200_matmul_pair call.
+template <typename T>
+class MatMulPairOp : public OpKernel {
+ public:
+  explicit MatMulPairOp(OpKernelConstruction* ctx) : OpKernel(ctx) {
+    for (int q = 0; q < 2; ++q) {
+      Product& p = p_[q];
+      const std::string sfx = q == 0 ? "0" : "1";
+      OP_REQUIRES_OK(ctx, ctx->GetAttr("transpose_a" + sfx, &p.ta));
+      OP_REQUIRES_OK(ctx, ctx->GetAttr("transpose_b" + sfx, &p.tb));
+      std::vector<std::string> fused;
+      OP_REQUIRES_OK(ctx, ctx->GetAttr("fused_ops" + sfx, &fused));
+      int64 num_args = 0;
+      OP_REQUIRES_OK(ctx, ctx->GetAttr("num_args" + sfx, &num_args));
+      if (fused.empty()) p.mode = kNone;
+      else if (fused == std::vector<std::string>{"BiasAdd"}) p.mode = kBias;
+      else if (fused == std::vector<std::string>{"BiasAdd", "Relu"}) p.mode = kBiasRelu;
+      else if (fused == std::vector<std::string>{"ReluGrad"}) p.mode = kReluGrad;
+      else
+        OP_REQUIRES(ctx, false, errors::InvalidArgument("Unsupported fused_ops for _MatMulPair"));
+      OP_REQUIRES(ctx, num_args == (p.mode == kNone ? 0 : 1),
+                  errors::InvalidArgument("_MatMulPair: one extra argument per fused product"));
+    }
+  }
+
+  void Compute(OpKernelContext* ctx) override {
+    int next = 0;
+    bool degenerate = false;
+    for (int q = 0; q < 2; ++q) {
+      Product& p = p_[q];
+      const Tensor& a = ctx->input(next);
+      const Tensor& b = ctx->input(next + 1);
+      p.arg = p.mode == kNone ? nullptr : &ctx->input(next + 2);
+      next += p.mode == kNone ? 2 : 3;
+      OP_REQUIRES(ctx, TensorShapeUtils::IsMatrix(a.shape()),
+                  errors::InvalidArgument("In[0] is not a matrix"));
+      OP_REQUIRES(ctx, TensorShapeUtils::IsMatrix(b.shape()),
+                  errors::InvalidArgument("In[1] is not a matrix"));
+      const int a_contract = p.ta ? 0 : 1;
+      const int b_contract = p.tb ? 1 : 0;
+      OP_REQUIRES(ctx, a.dim_size(a_contract) == b.dim_size(b_contract),
+                  errors::InvalidArgument("Matrix size-incompatible: In[0]: ",
+                                          a.shape().DebugString(), ", In[1]: ",
+                                          b.shape().DebugString()));
+      p.a = &a;
+      p.b = &b;
+      p.m = a.dim_size(1 - a_contract);
+      p.k = a.dim_size(a_contract);
+      p.n = b.dim_size(1 - b_contract);
+      if (p.mode == kReluGrad) {
+        OP_REQUIRES(ctx, p.arg->shape() == TensorShape({p.m, p.n}),
+                    errors::InvalidArgument("Inputs must have the same size"));
+      } else if (p.mode != kNone) {
+        OP_REQUIRES(ctx, TensorShapeUtils::IsVector(p.arg->shape()),
+                    errors::InvalidArgument("Biases must be 1D: ", p.arg->shape().DebugString()));
+        OP_REQUIRES(ctx, p.arg->dim_size(0) == p.n,
+                    errors::InvalidArgument("Must provide as many biases as the last dimension of "
+                                            "the input tensor: ", p.arg->shape().DebugString(),
+                                            " vs. ", TensorShape({p.m, p.n}).DebugString()));
+      }
+      OP_REQUIRES_OK(ctx, ctx->allocate_output(q, TensorShape({p.m, p.n}), &p.out));
+      degenerate = degenerate || p.out->NumElements() == 0 || p.k == 0;
+    }
+    void* stream = GetCudaStream(ctx);
+    if (degenerate) {  // an empty output or k == 0: each product on its own, as its op does it
+      for (const Product& p : p_) RunOne(ctx, p, stream);
+      return;
+    }
+    const Product &p0 = p_[0], &p1 = p_[1];
+    const size_t ws_bytes =
+        b200_matmul_pair_workspace_bytes(AbiType<T>::v, p0.m, p0.n, p0.k, p1.m, p1.n, p1.k);
+    Tensor scratch;
+    if (ws_bytes > 0)
+      OP_REQUIRES_OK(ctx, ctx->allocate_temp(DT_UINT8, TensorShape({static_cast<int64>(ws_bytes)}),
+                                             &scratch));
+    OP_REQUIRES_OK(ctx, FromAbi(b200_matmul_pair(
+                                    AbiType<T>::v, p0.a->raw_data(), p0.b->raw_data(),
+                                    p0.out->raw_data(), p0.m, p0.n, p0.k, p0.ta, p0.tb, p0.bias(),
+                                    p0.mode == kBiasRelu, p0.features(), p1.a->raw_data(),
+                                    p1.b->raw_data(), p1.out->raw_data(), p1.m, p1.n, p1.k, p1.ta,
+                                    p1.tb, p1.bias(), p1.mode == kBiasRelu, p1.features(),
+                                    ws_bytes ? scratch.raw_data() : nullptr, ws_bytes, stream),
+                                "Blas GEMM launch failed"));
+  }
+
+ private:
+  enum Mode { kNone, kBias, kBiasRelu, kReluGrad };
+  struct Product {
+    bool ta = false, tb = false;
+    Mode mode = kNone;
+    const Tensor *a = nullptr, *b = nullptr, *arg = nullptr;
+    Tensor* out = nullptr;
+    int64 m = 0, n = 0, k = 0;
+    const void* bias() const { return mode == kBias || mode == kBiasRelu ? arg->raw_data() : nullptr; }
+    const void* features() const { return mode == kReluGrad ? arg->raw_data() : nullptr; }
+  };
+
+  static void RunOne(OpKernelContext* ctx, const Product& p, void* stream) {
+    if (p.out->NumElements() == 0) return;
+    void* c = p.out->raw_data();
+    if (p.k == 0) {  // product is zero: run the tail on a zero matrix, op by op
+      OP_REQUIRES_OK(ctx, FromAbi(b200_memset_async(c, 0, p.out->TotalBytes(), stream),
+                                  "_MatMulPair zero fill"));
+      if (p.bias())
+        OP_REQUIRES_OK(ctx, FromAbi(b200_bias_add(AbiType<T>::v, c, p.bias(), c, p.m, p.n, stream),
+                                    "BiasAdd"));
+      if (p.mode == kBiasRelu)
+        OP_REQUIRES_OK(ctx, FromAbi(b200_relu(AbiType<T>::v, c, c, p.m * p.n, stream), "Relu"));
+      return;
+    }
+    const size_t ws_bytes =
+        p.mode == kReluGrad ? 0 : b200_matmul_workspace_bytes(AbiType<T>::v, p.m, p.n, p.k);
+    Tensor scratch;
+    if (ws_bytes > 0)
+      OP_REQUIRES_OK(ctx, ctx->allocate_temp(DT_UINT8, TensorShape({static_cast<int64>(ws_bytes)}),
+                                             &scratch));
+    OP_REQUIRES_OK(ctx, FromAbi(b200_fused_matmul_ws(
+                                    AbiType<T>::v, p.a->raw_data(), p.b->raw_data(), c, p.m, p.n,
+                                    p.k, p.ta, p.tb, p.bias(), p.mode == kBiasRelu, p.features(),
+                                    ws_bytes ? scratch.raw_data() : nullptr, ws_bytes, stream),
+                                "Blas GEMM launch failed"));
+  }
+
+  Product p_[2];
+};
+
 #define REGISTER_GPU(T)                                                                        \
   REGISTER_KERNEL_BUILDER(Name("MatMul").Device(DEVICE_GPU).TypeConstraint<T>("T"),            \
                           MatMulOp<T>);                                                        \
   REGISTER_KERNEL_BUILDER(Name("BatchMatMul").Device(DEVICE_GPU).TypeConstraint<T>("T"),       \
                           BatchMatMulOp<T>);                                                   \
   REGISTER_KERNEL_BUILDER(Name("_FusedMatMul").Device(DEVICE_GPU).TypeConstraint<T>("T"),      \
-                          FusedMatMulOp<T>);
+                          FusedMatMulOp<T>);                                               \
+  REGISTER_KERNEL_BUILDER(Name("_MatMulPair").Device(DEVICE_GPU).TypeConstraint<T>("T"),       \
+                          MatMulPairOp<T>);
 REGISTER_B200_FLOAT_TYPES(REGISTER_GPU)
 #undef REGISTER_GPU
 

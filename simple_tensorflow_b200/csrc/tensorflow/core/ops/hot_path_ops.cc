@@ -26,6 +26,18 @@ REGISTER_OP("_FusedMatMul")
     .Attr("transpose_a: bool = false").Attr("transpose_b: bool = false")
     .Attr("fused_ops: list(string)");
 
+// Executor-internal (DirectSession::FuseSiblingMatMuls): two independent MatMul / _FusedMatMul
+// products, each with the inputs and attrs of a _FusedMatMul (a plain MatMul has num_args = 0 and
+// no fused_ops), computed by one persistent GEMM launch.
+REGISTER_OP("_MatMulPair")
+    .Input("a0: T").Input("b0: T").Input("args0: num_args0 * T")
+    .Input("a1: T").Input("b1: T").Input("args1: num_args1 * T")
+    .Output("product0: T").Output("product1: T")
+    .Attr("T: {float, bfloat16}").Attr("num_args0: int >= 0").Attr("num_args1: int >= 0")
+    .Attr("transpose_a0: bool = false").Attr("transpose_b0: bool = false")
+    .Attr("transpose_a1: bool = false").Attr("transpose_b1: bool = false")
+    .Attr("fused_ops0: list(string)").Attr("fused_ops1: list(string)");
+
 REGISTER_OP("BatchMatMul")
     .Input("x: T").Input("y: T").Output("output: T")
     .Attr("T: {half, float, double, int32, complex64, complex128, bfloat16}")
