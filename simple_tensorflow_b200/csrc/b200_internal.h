@@ -50,7 +50,6 @@ struct GemmArgs {
   long long strideA, strideB, strideC;  // batch strides (elements)
   bool a_mn_major;           // A stored as [K,M] (transpose_a)
   bool b_mn_major;           // B stored as [K,N] (i.e. NOT transpose_b)
-  int force_bn;              // 0 = auto
   void* workspace;           // optional device scratch enabling split-K (may be null)
   size_t workspace_bytes;
   // fused epilogue (tcgen05 path only; all optional)

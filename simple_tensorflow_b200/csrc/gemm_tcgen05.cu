@@ -12,16 +12,18 @@
 //
 // CTA layout (192 threads, one CTA per SM, persistent over output tiles):
 //   warp 0      : TMA producer  (cp.async.bulk.tensor -> 128B-swizzled smem ring, mbarrier tx)
-//   warp 1      : TMEM allocator + single-thread tcgen05.mma issuer
-//   warps 2..5  : epilogue (tcgen05.ld TMEM -> registers -> 128-bit global stores)
+//   warp 1      : TMEM allocator + tcgen05.mma issuer (the whole warp runs the loop, one elected
+//                 lane issues each instruction)
+//   warps 2..5  : epilogue (tcgen05.ld TMEM -> registers -> fused tail -> 128B-swizzled smem
+//                 staging -> TMA store; direct global stores for outputs TMA cannot address)
 // Pipelines: smem full/empty ring (kStages), TMEM accumulator full/empty (2 stages) so the
-// epilogue of tile i overlaps the main loop of tile i+1.
+// epilogue of tile i overlaps the main loop of tile i+1.  Split-K partials go to an fp32 scratch
+// buffer and are summed in ascending split order by a second, ordered reduction kernel.
 #include "b200_ptx.cuh"
 #include "b200_internal.h"
 
 #include <cuda_bf16.h>
 #include <algorithm>
-#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -83,12 +85,6 @@ struct GemmShape {
   int splits;         // split-K factor (1 = none)
   int kb_per_split;   // K blocks per split
   float* partial;     // [splits][batch][M][N] fp32 partial sums when splits > 1
-  // In-kernel split-K reduction (splits > 1): per-tile arrive / depart counters.  Every epilogue
-  // warp that has stored its partial rows arrives; once all splits of a tile have arrived the
-  // warps add the partials (ascending split order: deterministic) for their share of the rows
-  // and write C, so no second kernel and no second pass over the launch boundary is needed.
-  // nullptr: partials are left for splitk_reduce_kernel.
-  unsigned int* tickets;
   int a_map4d, b_map4d;  // MN-major operand described by a 4-D map: one TMA per stage
   // implicit-GEMM convolution A operand (conv_a != 0): K blocks enumerate (filter tap, channel block)
   int conv_a, cv_OW, cv_OH, cv_sh, cv_sw, cv_pt, cv_pl, cv_S, cv_C, cv_cblocks, cv_taps;
@@ -111,8 +107,6 @@ __device__ __forceinline__ void trace_mark(const GemmShape& s, int slot, bool la
     s.trace[slot] = t;
   }
 }
-
-__device__ __forceinline__ bool partial_out_tile(const GemmShape& s) { return s.splits > 1; }
 
 // One GEMM of a launch: operand maps, output (or partial-buffer) store map, ReluGrad-feature map.
 template <typename TOut>
@@ -177,39 +171,6 @@ template <typename TOut>
 __host__ __device__ constexpr int nvals_max() {
   return kSwizzleBytes / (int)sizeof(TOut);
 }
-template <typename TOut, int BN>
-__host__ __device__ constexpr int partial_out_iters() {
-  return BN / 32;
-}
-struct GemmShape;
-__device__ __forceinline__ bool partial_out_tile(const GemmShape& s);
-
-constexpr int kSplitKSlots = 16, kSplitKMaxTiles = 1024;
-// [slot][0..kMaxTiles) arrivals, [slot][kMaxTiles..2*kMaxTiles) departures; zero at rest (the last
-// warp to depart from a tile resets both), one slot per launch in rotation so that launches on
-// different streams of a device never share counters.
-__device__ unsigned int g_splitk_tickets[kSplitKSlots][2 * kSplitKMaxTiles];
-
-__device__ __forceinline__ unsigned int ld_acquire_gpu_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void store_out4(float* dst, const float4& a) {
-  *reinterpret_cast<float4*>(dst) = a;
-}
-__device__ __forceinline__ void store_out4(__nv_bfloat16* dst, const float4& a) {
-  __nv_bfloat162 lo = __floats2bfloat162_rn(a.x, a.y), hi = __floats2bfloat162_rn(a.z, a.w);
-  uint2 p;
-  p.x = *reinterpret_cast<uint32_t*>(&lo);
-  p.y = *reinterpret_cast<uint32_t*>(&hi);
-  *reinterpret_cast<uint2*>(dst) = p;
-}
-__device__ __forceinline__ void store_out1(float* dst, float a) { *dst = a; }
-__device__ __forceinline__ void store_out1(__nv_bfloat16* dst, float a) {
-  *dst = __float2bfloat16_rn(a);
-}
-
 // TIn: operand element type (float -> tf32 MMA, bf16 -> f16-kind MMA); TOut: stored type.
 // (kAMN, kBMN): operand majorness of problem 0; (kAMN1, kBMN1): that of problem 1 when kNP = 2.
 // Each problem's majorness stays a compile-time constant: every role selects the problem of a
@@ -578,8 +539,8 @@ gemm_tcgen05_kernel(const __grid_constant__ GemmParams<TOut, kNP> P) {
       // Bias slice of this tile -> this warp's (otherwise unused) feature staging, also ahead of
       // the accumulator: the per-chunk broadcast reads then hit smem instead of exposing an L2
       // round trip per chunk.
-      const bool bias_smem = s.bias != nullptr && s.bias_vec && !partial_out_tile(s) &&
-                             !feat_on && n0 + BN <= s.N;
+      const bool bias_smem = s.bias != nullptr && s.bias_vec && s.splits == 1 && !feat_on &&
+                             n0 + BN <= s.N;
       if (bias_smem) {
         const uint4* bsrc = reinterpret_cast<const uint4*>(static_cast<const TOut*>(s.bias) + n0);
         uint4* bdst = reinterpret_cast<uint4*>(my_feat);
@@ -596,8 +557,6 @@ gemm_tcgen05_kernel(const __grid_constant__ GemmParams<TOut, kNP> P) {
       // split-K: fp32 partial tile, dense [split][batch][M][N]
       float* prow = s.partial + (((long long)split * s.batch + b) * s.M + row) * (long long)s.N;
       const bool pvec = (s.N & 3) == 0;
-      constexpr int kIters = partial_out_iters<TOut, BN>();
-      (void)kIters;
       const int cols_per_iter = partial_out ? 32 : kEpiCols;
       const int iters = BN / cols_per_iter;
 #pragma unroll 1
@@ -765,103 +724,6 @@ gemm_tcgen05_kernel(const __grid_constant__ GemmParams<TOut, kNP> P) {
       if (++acc == 2) {
         acc = 0;
         acc_phase ^= 1;
-      }
-      if (partial_out && s.tickets != nullptr) {
-        // ---- in-kernel split-K reduction.  (1) publish this warp's partial rows
-        unsigned int* arrive = s.tickets + tile;
-        unsigned int* depart = s.tickets + kSplitKMaxTiles + tile;
-        const unsigned int expected = (unsigned int)s.splits * kCtas * 4u;
-        if (s.tma_store) {
-          if (lane == 0) {
-            tma_store_wait<0>();  // the bulk stores have been performed
-            asm volatile("fence.proxy.async;" ::: "memory");  // async-proxy writes -> generic
-          }
-          stores_in_flight = 0;
-        }
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) {
-          atomicAdd(arrive, 1u);
-          // (2) all splits of this tile have published (every CTA of the grid is resident: the
-          // grid never exceeds one CTA per SM, see launch_gemm)
-          while (ld_acquire_gpu_u32(arrive) < expected) {
-          }
-        }
-        __syncwarp();
-        // (3) this warp reduces rows split, split + splits, ... of its 32-row group over all
-        // splits in ascending order and writes C (coalesced: a warp covers 128 columns per access)
-        const bool n4 = (s.N & 3) == 0 && (s.ldc & 3) == 0 && (s.strideC & 3) == 0 &&
-                        ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
-        const long long per_split = (long long)s.batch * s.M * s.N;
-        if (n4) {
-          // Vector v of this warp = (row j = split + (v / kVecPerRow) * splits, 128-column group
-          // v % kVecPerRow).  kInFlight vectors x up to 4 splits of independent 16-byte loads are
-          // issued before the first add, so the L2 round trips overlap; the adds stay in
-          // ascending split order.
-          constexpr int kVecPerRow = BN >= 128 ? BN / 128 : 1;
-          constexpr int kInFlight = 4;
-          const int my_rows = split < 32 ? (32 - split + s.splits - 1) / s.splits : 0;
-          const int nvec = my_rows * kVecPerRow;
-          for (int v0 = 0; v0 < nvec; v0 += kInFlight) {
-            float4 a[kInFlight];
-            const float* src[kInFlight];
-            TOut* dst[kInFlight];
-            bool on[kInFlight];
-#pragma unroll
-            for (int u = 0; u < kInFlight; ++u) {
-              const int v = v0 + u;
-              const int j = split + (v / kVecPerRow) * s.splits;
-              const int r = row0 + j;
-              const int col = n0 + ((v % kVecPerRow) * 32 + lane) * 4;
-              on[u] = v < nvec && r < s.M && col < s.N && (BN >= 128 || lane * 4 < BN);
-              src[u] = s.partial + ((long long)b * s.M + r) * (long long)s.N + col;
-              dst[u] = C + (long long)b * s.strideC + (long long)r * s.ldc + col;
-              a[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-            for (int sp0 = 0; sp0 < s.splits; sp0 += 4) {
-              float4 t[kInFlight][4];
-#pragma unroll
-              for (int u = 0; u < kInFlight; ++u)
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                  if (on[u] && sp0 + q < s.splits)
-                    t[u][q] = __ldcg(reinterpret_cast<const float4*>(src[u] + (sp0 + q) * per_split));
-#pragma unroll
-              for (int u = 0; u < kInFlight; ++u)
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                  if (on[u] && sp0 + q < s.splits) {
-                    a[u].x += t[u][q].x;
-                    a[u].y += t[u][q].y;
-                    a[u].z += t[u][q].z;
-                    a[u].w += t[u][q].w;
-                  }
-            }
-#pragma unroll
-            for (int u = 0; u < kInFlight; ++u)
-              if (on[u]) store_out4(dst[u], a[u]);
-          }
-        } else {
-          for (int j = split; j < 32; j += s.splits) {
-            const int r = row0 + j;
-            if (r >= s.M) break;
-            const float* prow0 = s.partial + ((long long)b * s.M + r) * (long long)s.N;
-            TOut* crow_r = C + (long long)b * s.strideC + (long long)r * s.ldc;
-            for (int col = n0 + lane; col < n0 + BN && col < s.N; col += 32) {
-              float a = __ldcg(prow0 + col);
-              for (int sp = 1; sp < s.splits; ++sp) a += __ldcg(prow0 + sp * per_split + col);
-              store_out1(crow_r + col, a);
-            }
-          }
-        }
-        // (4) depart; the last warp out of the tile leaves both counters at zero
-        __syncwarp();
-        if (lane == 0) {
-          if (atomicAdd(depart, 1u) == expected - 1u) {
-            *depart = 0u;
-            *arrive = 0u;
-          }
-        }
       }
     });
     if (warp == 2 && lane == 0) trace_mark(P.p[0].s, 6);
@@ -1098,7 +960,6 @@ static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* 
   CUtensorMap& mb = pr.tmapB;
   int rc;
   // A: logical [M,K]; stored [M,K] (K-major) or [K,M] (MN-major).  Box = one CTA's 128 rows.
-  static const bool no_map4d = getenv("B200TF_GEMM_NO_MAP4D") != nullptr;
   bool a4 = false, b4 = false;
   if (g.conv_a) {
     if (kAMN)  // filter gradient: boxes of BK pixels x one 128-byte channel chunk
@@ -1108,8 +969,7 @@ static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* 
   } else if (!kAMN)
     rc = encode_operand_map(&ma, Tr::kTmaType, sizeof(TIn), g.a, g.M, g.K, g.lda, g.batch,
                             g.strideA, Tr::kBK, kBM, false);
-  else if (!no_map4d &&
-           (a4 = encode_mn_major_map4d(&ma, Tr::kTmaType, sizeof(TIn), g.a, g.K, g.M, g.lda,
+  else if ((a4 = encode_mn_major_map4d(&ma, Tr::kTmaType, sizeof(TIn), g.a, g.K, g.M, g.lda,
                                        g.batch, g.strideA, kChunk, Tr::kBK, kBM / kChunk)))
     rc = B200_OK;
   else
@@ -1120,8 +980,7 @@ static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* 
   if (!kBMN)
     rc = encode_operand_map(&mb, Tr::kTmaType, sizeof(TIn), g.b, g.N, g.K, g.ldb, g.batch,
                             g.strideB, Tr::kBK, kBNLocal, false);
-  else if (!no_map4d &&
-           (b4 = encode_mn_major_map4d(&mb, Tr::kTmaType, sizeof(TIn), g.b, g.K, g.N, g.ldb,
+  else if ((b4 = encode_mn_major_map4d(&mb, Tr::kTmaType, sizeof(TIn), g.b, g.K, g.N, g.ldb,
                                        g.batch, g.strideB, kChunk, Tr::kBK, kBNLocal / kChunk)))
     rc = B200_OK;
   else
@@ -1173,10 +1032,7 @@ static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* 
   s.ld_features = (int)g.ld_features;
   CUtensorMap& mc = pr.tmapC;
   memset(&mc, 0, sizeof(mc));
-  static const bool no_tma_store = getenv("B200TF_GEMM_DIRECT_STORE") != nullptr;
-  if (no_tma_store)
-    s.tma_store = 0;
-  else if (splits > 1)
+  if (splits > 1)
     s.tma_store = encode_store_map(&mc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, g.workspace, g.M, g.N,
                                    g.N, (long long)splits * g.batch, g.M * g.N);
   else
@@ -1193,54 +1049,6 @@ static int prepare_problem(const GemmArgs& g, GemmProblem<TOut>& pr, long long* 
                                   g.ld_features, 1, g.M * g.ld_features);
   s.bias_vec = g.bias && (reinterpret_cast<uintptr_t>(g.bias) & 15) == 0;
   s.trace = nullptr;
-  s.tickets = nullptr;
-  return B200_OK;
-}
-
-// One persistent launch of `kern` over grid_units CTAs (pairs): cluster and PDL attributes,
-// the one-time shared-memory opt-in, and the B200TF_KERNEL_TIMES bracket.
-template <typename TOut, int kNP>
-static int launch_persistent(void (*kern)(GemmParams<TOut, kNP>), bool& attr_set,
-                             const GemmParams<TOut, kNP>& P, int grid_units, int ctas, size_t smem,
-                             bool pdl, cudaStream_t stream) {
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
-    if (e != cudaSuccess) {
-      set_last_error("cudaFuncSetAttribute(smem=%zu): %s", smem, cudaGetErrorString(e));
-      return B200_INTERNAL;
-    }
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid_units * ctas);
-  cfg.blockDim = dim3(kGemmThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (ctas > 1) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = ctas;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  if (pdl) {  // prologue overlaps the predecessor's tail; the kernel pdl_wait()s before global I/O
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, P);
-  if (ktok) kernel_times_end(ktok, stream, reinterpret_cast<const void*>(kern));
-  if (e != cudaSuccess) {
-    set_last_error("gemm_tcgen05 launch: %s", cudaGetErrorString(e));
-    cudaGetLastError();
-    return B200_INTERNAL;
-  }
   return B200_OK;
 }
 
@@ -1261,8 +1069,7 @@ static int launch_splitk_reduce(const GemmArgs& g, const GemmShape& s, bool pdl,
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl && !prof ? 1 : 0;
-  static const bool generic_only = getenv("B200TF_SPLITK_REDUCE_GENERIC") != nullptr;
-  const bool flat = !generic_only && (s.N & 3) == 0 && s.ldc == s.N &&
+  const bool flat = (s.N & 3) == 0 && s.ldc == s.N &&
                     (g.batch == 1 || (long long)s.strideC == (long long)s.M * s.N) &&
                     splits >= 2 && splits <= 16 &&
                     (reinterpret_cast<uintptr_t>(s.partial) & 15) == 0 &&
@@ -1320,16 +1127,34 @@ static int launch_splitk_reduce(const GemmArgs& g, const GemmShape& s, bool pdl,
   return B200_OK;
 }
 
-template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas>
-static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
-  GemmParams<TOut, 1> P;
+// One persistent launch over kNP problems, then one ordered reduction pass per split problem.
+// kNP = 1: one GEMM.  kNP = 2: a dense layer's input gradient dX = dY * W^T (slot 0: both operands
+// K-major) and weight gradient dW = X^T * dY (slot 1: both MN-major) with BN-wide pair tiles.  Each
+// problem keeps the split plan, tile order and fused tail of its own launch, so every output is
+// bit-identical to it; the problem whose items are longer comes first in the work list, so that
+// the short items fill the tail.  The pair counts as one GEMM launch with the summed FLOPs.
+template <typename TIn, typename TOut, bool kAMN, bool kBMN, int BN, int kCtas, int kNP = 1,
+          bool kAMN1 = false, bool kBMN1 = false>
+static int launch_gemm(const GemmArgs* const (&g)[kNP], cudaStream_t stream) {
+  constexpr auto kern = gemm_tcgen05_kernel<TIn, TOut, kAMN, kBMN, BN, kCtas, kNP, kAMN1, kBMN1>;
+  constexpr size_t smem = gemm_smem_bytes<BN, kCtas>();
+  GemmParams<TOut, kNP> P;
   memset(&P, 0, sizeof(P));
-  long long tiles = 0;
-  int rc = prepare_problem<TIn, TOut, kAMN, kBMN, BN, kCtas>(g, P.p[0], &tiles);
-  if (rc) return rc;
-  GemmShape& s = P.p[0].s;
-  const int splits = s.splits;
-  const int units = sm_count() / kCtas;
+  long long work[kNP], total_work = 0;
+  double flops = 0.0;
+  for (int i = 0; i < kNP; ++i) {
+    long long tiles = 0;
+    const int rc = i == 0 ? prepare_problem<TIn, TOut, kAMN, kBMN, BN, kCtas>(*g[0], P.p[0], &tiles)
+                          : prepare_problem<TIn, TOut, kAMN1, kBMN1, BN, kCtas>(*g[i], P.p[i], &tiles);
+    if (rc) return rc;
+    work[i] = tiles * P.p[i].s.splits;
+    total_work += work[i];
+    flops += 2.0 * (double)g[i]->M * (double)g[i]->N * (double)g[i]->K * g[i]->batch;
+  }
+  if constexpr (kNP == 2) {
+    P.first = P.p[1].s.kb_per_split > P.p[0].s.kb_per_split ? 1 : 0;
+    P.first_work = (int)work[P.first];
+  }
   static const bool trace_on = getenv("B200TF_GEMM_TRACE") != nullptr;
   static unsigned long long* trace_buf = nullptr;
   if (trace_on) {
@@ -1337,114 +1162,84 @@ static int launch_gemm(const GemmArgs& g, cudaStream_t stream) {
     if (trace_buf != nullptr) {
       cudaMemsetAsync(trace_buf, 0, 16 * sizeof(unsigned long long), stream);
       cudaStreamSynchronize(stream);
-      s.trace = trace_buf;
+      for (int i = 0; i < kNP; ++i) P.p[i].s.trace = trace_buf;
     }
   }
-  const long long work = tiles * splits;
-  const int grid_units = (int)(work < units ? work : units);
-  // In-kernel reduction (B200TF_SPLITK_INKERNEL=1) needs every (split, tile) work item on its own
-  // resident CTA (pair), so that waiting for the other splits of a tile cannot deadlock:
-  // plan_splits guarantees work <= units.  Measured on the MLP's dW GEMM (1024x1024x4096, 4
-  // splits): 26.7 us in-kernel vs 26.6 us with the separate ordered pass, step time unchanged --
-  // the wait for the slowest split plus the L2 round trips of the reduction cost what the second
-  // launch costs -- so the simpler two-kernel form stays the default (profiles/r02_notes.md).
-  static const bool inkernel_reduce = getenv("B200TF_SPLITK_INKERNEL") != nullptr;
-  if (splits > 1 && inkernel_reduce && !g.bias && work <= units && tiles <= kSplitKMaxTiles) {
-    static unsigned int* ticket_base[64] = {nullptr};
-    static std::atomic<unsigned> next_slot{0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64) {
-      if (ticket_base[dev] == nullptr) {
-        void* sym = nullptr;
-        if (cudaGetSymbolAddress(&sym, g_splitk_tickets) == cudaSuccess)
-          ticket_base[dev] = static_cast<unsigned int*>(sym);
-        else
-          cudaGetLastError();
-      }
-      if (ticket_base[dev] != nullptr)
-        s.tickets = ticket_base[dev] +
-                    (size_t)(next_slot.fetch_add(1) % kSplitKSlots) * 2 * kSplitKMaxTiles;
+  static bool attr_set = false;  // per template instantiation
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) {
+      set_last_error("cudaFuncSetAttribute(smem=%zu): %s", smem, cudaGetErrorString(e));
+      return B200_INTERNAL;
     }
+    attr_set = true;
   }
   const bool prof = profile_enabled();
-  if (prof) profile_gemm_launch_begin(stream);
   const bool pdl = pdl_enabled();
-  static bool attr_set = false;  // per template instantiation
-  rc = launch_persistent<TOut, 1>(gemm_tcgen05_kernel<TIn, TOut, kAMN, kBMN, BN, kCtas>, attr_set,
-                                  P, grid_units, kCtas, gemm_smem_bytes<BN, kCtas>(), pdl, stream);
-  if (rc) return rc;
-  if (prof) profile_gemm_launch_end(stream, 2.0 * (double)g.M * (double)g.N * (double)g.K * g.batch);
-  if (s.trace != nullptr) {  // debug: phase boundaries, ns since the first CTA entered the kernel
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)std::min<long long>(total_work, sm_count() / kCtas) * kCtas);
+  cfg.blockDim = dim3(kGemmThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[2];
+  int na = 0;
+  if (kCtas > 1) {
+    attr[na].id = cudaLaunchAttributeClusterDimension;
+    attr[na].val.clusterDim.x = kCtas;
+    attr[na].val.clusterDim.y = 1;
+    attr[na].val.clusterDim.z = 1;
+    ++na;
+  }
+  if (pdl) {  // prologue overlaps the predecessor's tail; the kernel pdl_wait()s before global I/O
+    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
+  }
+  cfg.attrs = attr;
+  cfg.numAttrs = na;
+  if (prof) profile_gemm_launch_begin(stream);
+  void* ktok = kernel_times_enabled() ? kernel_times_begin(stream) : nullptr;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, P);
+  if (ktok) kernel_times_end(ktok, stream, reinterpret_cast<const void*>(kern));
+  if (e != cudaSuccess) {
+    set_last_error("gemm_tcgen05 launch: %s", cudaGetErrorString(e));
+    cudaGetLastError();
+    return B200_INTERNAL;
+  }
+  if (prof) profile_gemm_launch_end(stream, flops);
+  if (P.p[0].s.trace != nullptr) {  // debug: phase boundaries, ns since the first CTA entered
     unsigned long long t[16];
     cudaStreamSynchronize(stream);
-    cudaMemcpy(t, s.trace, sizeof(t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(t, P.p[0].s.trace, sizeof(t), cudaMemcpyDeviceToHost);
     fprintf(stderr,
-            "[gemm trace] %dx%dx%d BN=%d ctas=%d splits=%d: prologue %llu | pdl_wait %llu | first "
-            "operands %llu | mainloop issued %llu | accumulator ready %llu | epilogue stored %llu | "
-            "stores drained %llu | exit %llu | last CTA entry %lld exit %lld (ns since entry)\n",
-            g.M, g.N, g.K, BN, kCtas, splits, t[1] - t[0], t[2] - t[0], t[3] - t[0], t[4] - t[0],
-            t[5] - t[0], t[6] - t[0], t[7] - t[0], t[8] - t[0], (long long)(t[9] - t[0]),
-            (long long)(t[10] - t[0]));
+            "[gemm trace] %lldx%lldx%lld BN=%d ctas=%d problems=%d splits=%d: prologue %llu | "
+            "pdl_wait %llu | first operands %llu | mainloop issued %llu | accumulator ready %llu | "
+            "epilogue stored %llu | stores drained %llu | exit %llu | last CTA entry %lld exit "
+            "%lld (ns since entry)\n",
+            g[0]->M, g[0]->N, g[0]->K, BN, kCtas, kNP, P.p[0].s.splits, t[1] - t[0], t[2] - t[0],
+            t[3] - t[0], t[4] - t[0], t[5] - t[0], t[6] - t[0], t[7] - t[0], t[8] - t[0],
+            (long long)(t[9] - t[0]), (long long)(t[10] - t[0]));
   }
   note_launch();
-  if (splits > 1 && s.tickets == nullptr) {
-    rc = launch_splitk_reduce<TOut>(g, s, pdl, prof, stream);
-    if (rc) return rc;
-  }
-  return check_launch("gemm_tcgen05");
-}
-
-// A dense layer's input gradient dX = dY * W^T (slot 0: both operands K-major) and weight gradient
-// dW = X^T * dY (slot 1: both MN-major) in one persistent launch of BN-wide pair tiles.  Each
-// problem keeps the split plan, tile order and fused tail of its own launch, so every output is
-// bit-identical to it; split problems keep their own reduction pass afterwards.  The problem
-// whose items are longer comes first in the work list, so that the short items fill the tail.
-template <typename TIn, typename TOut, int BN>
-static int launch_gemm_pair(const GemmArgs& g0, const GemmArgs& g1, cudaStream_t stream) {
-  constexpr int kCtas = 2;
-  GemmParams<TOut, 2> P;
-  memset(&P, 0, sizeof(P));
-  long long tiles0 = 0, tiles1 = 0;
-  int rc = prepare_problem<TIn, TOut, false, false, BN, kCtas>(g0, P.p[0], &tiles0);
-  if (rc) return rc;
-  rc = prepare_problem<TIn, TOut, true, true, BN, kCtas>(g1, P.p[1], &tiles1);
-  if (rc) return rc;
-  const long long work0 = tiles0 * P.p[0].s.splits, work1 = tiles1 * P.p[1].s.splits;
-  P.first = P.p[1].s.kb_per_split > P.p[0].s.kb_per_split ? 1 : 0;
-  P.first_work = (int)(P.first ? work1 : work0);
-  const int units = sm_count() / kCtas;
-  const long long work = work0 + work1;
-  const int grid_units = (int)(work < units ? work : units);
-  const bool prof = profile_enabled();
-  if (prof) profile_gemm_launch_begin(stream);
-  const bool pdl = pdl_enabled();
-  static bool attr_set = false;  // per template instantiation
-  rc = launch_persistent<TOut, 2>(
-      gemm_tcgen05_kernel<TIn, TOut, false, false, BN, kCtas, 2, true, true>, attr_set, P,
-      grid_units, kCtas, gemm_smem_bytes<BN, kCtas>(), pdl, stream);
-  if (rc) return rc;
-  if (prof)
-    profile_gemm_launch_end(stream, 2.0 * ((double)g0.M * (double)g0.N * (double)g0.K +
-                                           (double)g1.M * (double)g1.N * (double)g1.K));
-  note_launch();
-  for (int i = 0; i < 2; ++i)
+  for (int i = 0; i < kNP; ++i)
     if (P.p[i].s.splits > 1) {
-      rc = launch_splitk_reduce<TOut>(i ? g1 : g0, P.p[i].s, pdl, prof, stream);
+      const int rc = launch_splitk_reduce<TOut>(*g[i], P.p[i].s, pdl, prof, stream);
       if (rc) return rc;
     }
-  return check_launch("gemm_tcgen05_pair");
+  return check_launch("gemm_tcgen05");
 }
 
 template <typename TIn, typename TOut, int BN, int kCtas>
 static int dispatch_major(const GemmArgs& g, cudaStream_t stream) {
+  const GemmArgs* const gs[1] = {&g};
   if (!g.a_mn_major && !g.b_mn_major)
-    return launch_gemm<TIn, TOut, false, false, BN, kCtas>(g, stream);
+    return launch_gemm<TIn, TOut, false, false, BN, kCtas>(gs, stream);
   if (!g.a_mn_major && g.b_mn_major)
-    return launch_gemm<TIn, TOut, false, true, BN, kCtas>(g, stream);
+    return launch_gemm<TIn, TOut, false, true, BN, kCtas>(gs, stream);
   if (g.a_mn_major && !g.b_mn_major)
-    return launch_gemm<TIn, TOut, true, false, BN, kCtas>(g, stream);
-  return launch_gemm<TIn, TOut, true, true, BN, kCtas>(g, stream);
+    return launch_gemm<TIn, TOut, true, false, BN, kCtas>(gs, stream);
+  return launch_gemm<TIn, TOut, true, true, BN, kCtas>(gs, stream);
 }
 
 // Split-K plan shared by the launcher and gemm_workspace_bytes(): how many K splits a tiling
@@ -1464,18 +1259,7 @@ struct TileConfig {
   int ctas, bn;
 };
 static TileConfig choose_config(const GemmArgs& g) {
-  if (g.force_bn == 64) return {1, 64};
-  if (g.force_bn == 128) return {1, 128};
-  if (g.force_bn == 2128) return {2, 128};
-  if (g.force_bn == 2256) return {2, 256};
-  const char* env = getenv("B200TF_GEMM_CTAS");
-  const bool allow_pairs = !(env && env[0] == '1');
-  static const int pair_bn = [] {  // experiment switch: B200TF_GEMM_PAIR_BN=128 forces 256x128 pair tiles
-    const char* v = getenv("B200TF_GEMM_PAIR_BN");
-    return v ? atoi(v) : 0;
-  }();
-  if (allow_pairs && g.M >= 256 && g.N >= 128)
-    return {2, pair_bn == 128 ? 128 : (g.N >= 256 ? 256 : 128)};
+  if (g.M >= 256 && g.N >= 128) return {2, g.N >= 256 ? 256 : 128};
   if (g.N <= 64) return {1, 64};
   const long long t128 = ((g.M + kBM - 1) / kBM) * ((g.N + 127) / 128) * g.batch;
   if (t128 >= sm_count()) return {1, 128};
@@ -1550,12 +1334,13 @@ int gemm_tcgen05_pair(const GemmArgs& a, const GemmArgs& b, cudaStream_t stream)
     const int rc = gemm_tcgen05(a, stream);
     return rc ? rc : gemm_tcgen05(b, stream);
   }
+  const GemmArgs* const gs[2] = {&g0, &g1};
+  using bf16 = __nv_bfloat16;
   if (g0.dtype == B200_DT_FLOAT)
-    return c0.bn == 256 ? launch_gemm_pair<float, float, 256>(g0, g1, stream)
-                        : launch_gemm_pair<float, float, 128>(g0, g1, stream);
-  return c0.bn == 256
-             ? launch_gemm_pair<__nv_bfloat16, __nv_bfloat16, 256>(g0, g1, stream)
-             : launch_gemm_pair<__nv_bfloat16, __nv_bfloat16, 128>(g0, g1, stream);
+    return c0.bn == 256 ? launch_gemm<float, float, false, false, 256, 2, 2, true, true>(gs, stream)
+                        : launch_gemm<float, float, false, false, 128, 2, 2, true, true>(gs, stream);
+  return c0.bn == 256 ? launch_gemm<bf16, bf16, false, false, 256, 2, 2, true, true>(gs, stream)
+                      : launch_gemm<bf16, bf16, false, false, 128, 2, 2, true, true>(gs, stream);
 }
 
 }  // namespace b200

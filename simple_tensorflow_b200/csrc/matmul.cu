@@ -429,60 +429,15 @@ static int validate_gemm(const char* what, int dtype, const void* a, const void*
   return require_device(what);
 }
 
-}  // namespace b200
-
-using namespace b200;
-
-extern "C" {
-
-size_t b200_matmul_workspace_bytes(int dtype, int64_t m, int64_t n, int64_t k) {
-  return gemm_workspace_bytes(dtype, m, n, k, 1);
-}
-
-int b200_matmul(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n, int64_t k,
-                int transpose_a, int transpose_b, void* workspace, size_t workspace_bytes,
-                void* stream) {
-  int rc = validate_gemm("b200_matmul", dtype, a, b, c, m, n, k, 1);
-  if (rc) return rc;
-  GemmArgs g{};
-  g.dtype = dtype;
-  g.a = a;
-  g.b = b;
-  g.c = c;
-  g.M = m;
-  g.N = n;
-  g.K = k;
-  g.batch = 1;
-  g.lda = transpose_a ? m : k;
-  g.ldb = transpose_b ? k : n;
-  g.ldc = n;
-  g.strideA = m * k;
-  g.strideB = k * n;
-  g.strideC = m * n;
-  g.a_mn_major = transpose_a != 0;
-  g.b_mn_major = transpose_b == 0;
-  g.workspace = workspace;
-  g.workspace_bytes = workspace ? workspace_bytes : 0;
-  return gemm_dispatch(g, as_stream(stream));
-}
-
-int b200_fused_matmul(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n,
-                      int64_t k, int transpose_a, int transpose_b, const void* bias, int relu,
-                      const void* relu_grad_features, void* stream) {
-  return b200_fused_matmul_ws(dtype, a, b, c, m, n, k, transpose_a, transpose_b, bias, relu,
-                              relu_grad_features, nullptr, 0, stream);
-}
-
-}  // extern "C"
-
-namespace b200 {
-
-// Arguments of one (optionally fused) 2-D product, as b200_fused_matmul_ws takes them.
-static int fused_matmul_args(const char* what, int dtype, const void* a, const void* b, void* c,
-                             int64_t m, int64_t n, int64_t k, int transpose_a, int transpose_b,
-                             const void* bias, int relu, const void* relu_grad_features,
-                             void* workspace, size_t workspace_bytes, GemmArgs* out) {
-  int rc = validate_gemm(what, dtype, a, b, c, m, n, k, 1);
+// Arguments of one row-major product C[batch][m, n] = op(A) * op(B), validated under the name
+// `what`: an optional fused tail (bias, relu or relu-grad features) and optional scratch that lets
+// the product split K.
+static int product_args(const char* what, int dtype, const void* a, const void* b, void* c,
+                        int64_t batch, int64_t m, int64_t n, int64_t k, int transpose_a,
+                        int transpose_b, const void* bias, int relu,
+                        const void* relu_grad_features, void* workspace, size_t workspace_bytes,
+                        GemmArgs* out) {
+  int rc = validate_gemm(what, dtype, a, b, c, m, n, k, batch);
   if (rc) return rc;
   if (relu && relu_grad_features) {
     set_last_error("%s: relu and relu_grad_features are mutually exclusive", what);
@@ -496,7 +451,7 @@ static int fused_matmul_args(const char* what, int dtype, const void* a, const v
   g.M = m;
   g.N = n;
   g.K = k;
-  g.batch = 1;
+  g.batch = batch;
   g.lda = transpose_a ? m : k;
   g.ldb = transpose_b ? k : n;
   g.ldc = n;
@@ -535,16 +490,38 @@ static size_t align256(size_t x) { return (x + 255) & ~static_cast<size_t>(255);
 
 }  // namespace b200
 
+using namespace b200;
+
 extern "C" {
+
+size_t b200_matmul_workspace_bytes(int dtype, int64_t m, int64_t n, int64_t k) {
+  return gemm_workspace_bytes(dtype, m, n, k, 1);
+}
+
+int b200_matmul(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n, int64_t k,
+                int transpose_a, int transpose_b, void* workspace, size_t workspace_bytes,
+                void* stream) {
+  GemmArgs g;
+  const int rc = product_args("b200_matmul", dtype, a, b, c, 1, m, n, k, transpose_a, transpose_b,
+                              nullptr, 0, nullptr, workspace, workspace_bytes, &g);
+  return rc ? rc : fused_matmul(g, as_stream(stream));
+}
+
+int b200_fused_matmul(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n,
+                      int64_t k, int transpose_a, int transpose_b, const void* bias, int relu,
+                      const void* relu_grad_features, void* stream) {
+  return b200_fused_matmul_ws(dtype, a, b, c, m, n, k, transpose_a, transpose_b, bias, relu,
+                              relu_grad_features, nullptr, 0, stream);
+}
 
 int b200_fused_matmul_ws(int dtype, const void* a, const void* b, void* c, int64_t m, int64_t n,
                          int64_t k, int transpose_a, int transpose_b, const void* bias, int relu,
                          const void* relu_grad_features, void* workspace, size_t workspace_bytes,
                          void* stream) {
   GemmArgs g;
-  const int rc = fused_matmul_args("b200_fused_matmul", dtype, a, b, c, m, n, k, transpose_a,
-                                   transpose_b, bias, relu, relu_grad_features, workspace,
-                                   workspace_bytes, &g);
+  const int rc = product_args("b200_fused_matmul", dtype, a, b, c, 1, m, n, k, transpose_a,
+                              transpose_b, bias, relu, relu_grad_features, workspace,
+                              workspace_bytes, &g);
   return rc ? rc : fused_matmul(g, as_stream(stream));
 }
 
@@ -566,13 +543,13 @@ int b200_matmul_pair(int dtype, const void* a0, const void* b0, void* c0, int64_
   const size_t off1 = align256(ws0);
   void* w1 = workspace_bytes > off1 ? static_cast<char*>(workspace) + off1 : nullptr;
   GemmArgs g0, g1;
-  int rc = fused_matmul_args("b200_matmul_pair", dtype, a0, b0, c0, m0, n0, k0, transpose_a0,
-                             transpose_b0, bias0, relu0, relu_grad_features0, workspace,
-                             std::min(ws0, workspace_bytes), &g0);
+  int rc = product_args("b200_matmul_pair", dtype, a0, b0, c0, 1, m0, n0, k0, transpose_a0,
+                        transpose_b0, bias0, relu0, relu_grad_features0, workspace,
+                        std::min(ws0, workspace_bytes), &g0);
   if (rc) return rc;
-  rc = fused_matmul_args("b200_matmul_pair", dtype, a1, b1, c1, m1, n1, k1, transpose_a1,
-                         transpose_b1, bias1, relu1, relu_grad_features1, w1,
-                         w1 ? workspace_bytes - off1 : 0, &g1);
+  rc = product_args("b200_matmul_pair", dtype, a1, b1, c1, 1, m1, n1, k1, transpose_a1,
+                    transpose_b1, bias1, relu1, relu_grad_features1, w1,
+                    w1 ? workspace_bytes - off1 : 0, &g1);
   if (rc) return rc;
   const cudaStream_t s = as_stream(stream);
   if (use_tcgen05(g0) && use_tcgen05(g1)) return gemm_tcgen05_pair(g0, g1, s);
@@ -582,26 +559,10 @@ int b200_matmul_pair(int dtype, const void* a0, const void* b0, void* c0, int64_
 
 int b200_batch_matmul(int dtype, const void* x, const void* y, void* out, int64_t batch, int64_t m,
                       int64_t n, int64_t k, int adj_x, int adj_y, void* stream) {
-  int rc = validate_gemm("b200_batch_matmul", dtype, x, y, out, m, n, k, batch);
-  if (rc) return rc;
-  GemmArgs g{};
-  g.dtype = dtype;
-  g.a = x;
-  g.b = y;
-  g.c = out;
-  g.M = m;
-  g.N = n;
-  g.K = k;
-  g.batch = batch;
-  g.lda = adj_x ? m : k;
-  g.ldb = adj_y ? k : n;
-  g.ldc = n;
-  g.strideA = m * k;
-  g.strideB = k * n;
-  g.strideC = m * n;
-  g.a_mn_major = adj_x != 0;
-  g.b_mn_major = adj_y == 0;
-  return gemm_dispatch(g, as_stream(stream));
+  GemmArgs g;
+  const int rc = product_args("b200_batch_matmul", dtype, x, y, out, batch, m, n, k, adj_x, adj_y,
+                              nullptr, 0, nullptr, nullptr, 0, &g);
+  return rc ? rc : gemm_dispatch(g, as_stream(stream));
 }
 
 }  // extern "C"

@@ -169,3 +169,46 @@ def test_full_size_mlp_step_launches():
         for _ in range(3):
             sess.run(list(B.resident))
         assert sess.last_run_stats()["kernels_launched"] == 15
+
+
+def _degenerate_graph(case):
+    """Fetches and numpy results of a graph whose products have k == 0 or an empty output."""
+    rng = np.random.RandomState(5)
+    a, b = np.zeros((4, 0), np.float32), np.zeros((0, 3), np.float32)
+    if case == "matmul_k0":
+        return [tf.matmul(tf.constant(a), tf.constant(b))], [a @ b]
+    if case == "bias_relu_k0":  # _FusedMatMul: the tail runs on a zero product
+        bias = np.array([0.5, -0.25, 0.0], np.float32)
+        y = tf.relu(tf.bias_add(tf.matmul(tf.constant(a), tf.constant(b)), tf.constant(bias)))
+        return [y], [np.maximum(np.broadcast_to(bias, (4, 3)), 0)]
+    # _MatMulPair: X [0, 5] feeds X W (empty output) and dW = X^T dY (k == 0, zero-filled).  The
+    # constants come first: a product pairs only with one whose inputs exist at its place.
+    x, dy = np.zeros((0, 5), np.float32), np.zeros((0, 3), np.float32)
+    w = rng.uniform(-1, 1, (5, 3)).astype(np.float32)
+    X, Wt, DY = tf.constant(x), tf.constant(w), tf.constant(dy)
+    return [tf.matmul(X, Wt), tf.matmul(X, DY, transpose_a=True)], [x @ w, x.T @ dy]
+
+
+# case -> how many nodes fewer the fused graph runs than the op-by-op one
+DEGENERATE = {"matmul_k0": 0, "bias_relu_k0": 2, "pair": 1}
+
+
+@pytest.mark.parametrize("case", list(DEGENERATE))
+def test_session_degenerate_products_match_unfused(case, monkeypatch):
+    def run(disable):
+        if disable:
+            monkeypatch.setenv("B200TF_DISABLE_FUSION", "1")
+        else:
+            monkeypatch.delenv("B200TF_DISABLE_FUSION", raising=False)
+        tf.reset_default_graph()
+        fetches, want = _degenerate_graph(case)
+        with client.Session(tf.get_default_graph()) as sess:
+            return sess.run(fetches), want, sess.last_run_stats()["nodes_executed"]
+
+    got, want, nodes = run(disable=False)
+    ref, _, ref_nodes = run(disable=True)
+    assert ref_nodes - nodes == DEGENERATE[case]
+    for g, r, w in zip(got, ref, want):
+        assert g.shape == w.shape
+        np.testing.assert_array_equal(g, w)
+        np.testing.assert_array_equal(g.view(np.uint32), r.view(np.uint32))
